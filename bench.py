@@ -5,6 +5,7 @@
     python bench.py --impl reference --steps K --warmup W         # the UNMODIFIED reference's CPU path, same workload
     python bench.py --workload decode                             # config #5: KV-cached generation sweep, batch 1-1024
     python bench.py --workload bigram|singlehead|residual         # configs #1-#3: small-model train steps
+    python bench.py --steps K --warmup W --dump-outputs DIR       # also write the headline's outputs as DIR/*.npy
 
 One process per GPU (torchrun for N > 1, NCCL).  A "step" of the headline workload = forward + backward + gradient
 reduction + AdamW on one synthetic batch of 64 x 256 tokens per GPU (weak scaling), replayed from a CUDA graph.
@@ -22,6 +23,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 S = dict(vocab_size=80, embedding_dim=384, context_length=256, num_heads=6, num_layers=6, dropout=0.2,
@@ -169,12 +171,12 @@ def run_reference(args):
         return run_reference_decode(args)
     if args.workload in SMALL:
         kind, cfg, metric, wl = SMALL[args.workload], P, f"train_tokens_per_sec_{SMALL[args.workload]}", small_workload(args.workload)
-        steps, warmup = max(1, min(args.steps, 200)), max(1, min(args.warmup, 5))
+        warmup = max(1, min(args.warmup, 5))
     else:
         kind, cfg, metric, wl = "TransformerLM", S, METRIC, WORKLOAD
-        steps, warmup = max(1, min(args.steps, 5)), max(1, min(args.warmup, 2))  # ~4-8 s per 64x256 step on a host
+        warmup = max(1, min(args.warmup, 2))  # ~4-8 s per 64x256 step on a host
     B = cfg["batch_size"]
-    r = cpu_train_tokens_per_sec(kind, cfg, B, steps, warmup)
+    r = cpu_train_tokens_per_sec(kind, cfg, B, args.steps, warmup)
     sample = (f"{r['steps']} train steps (fwd+zero_grad+bwd+AdamW.step, src/train.py:143-151) of {B}x{cfg['context_length']} "
               f"tokens, fp32 torch CPU, {r['cores']} threads, "
               + ("the unmodified reference classes (oracle/_ref)" if r["kind"] == "reference" else "oracle port"))
@@ -211,6 +213,23 @@ def roofline_dominant(dev, pk):
             "kernel": "gemm_tc_kernel dgrad (A K-major, B MN-major, bf16 out) FFN1 dgrad 16384x384x1536, operands from HBM "
                       "(6 rotating sets); the instantiation with the largest share of the step",
             "peak_source": pk["src"] + " burst", "us_per_launch": us, "launches_timed": 5 * 4 * probes.R}
+
+
+def dump_train_outputs(out_dir, model, reducer, loss, rank):
+    """Write what the last step of the headline timed window hands its caller, so that two builds can be compared
+    output for output: the step's loss and every parameter after its AdamW update (fp32 masters under their reference
+    state_dict names, 43 MB for TransformerLM_scaled), as float32 out_dir/<name>.npy.  The fixed causal-mask buffers
+    are left out."""
+    if reducer is not None and getattr(reducer, "fused_optimizer", False):
+        reducer.sync_master()  # each rank updated only its own shard of the fp32 masters
+        torch.distributed.barrier()  # no rank starts its next step while a peer still reads its masters
+    if rank != 0:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array(loss, dtype=np.float32))
+    for name, t in model.state_dict().items():
+        if not name.endswith(".tril"):
+            np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def run_train(args):
@@ -275,6 +294,8 @@ def run_train(args):
         dt, loss = timed(pool_dev, sync_each=False)
     eager_launches = ops.launch_count() - n1
     clocks = cs.summary()
+    if args.dump_outputs:
+        dump_train_outputs(args.dump_outputs, model, reducer, loss, rank)
     dt_e2e, _ = timed(pool_host, sync_each=True)
     tokens = world * B * T * args.steps
     tps, tps_e2e = tokens / dt, tokens / dt_e2e
@@ -496,7 +517,13 @@ def main():
     ap.add_argument("--no-graph", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-kernel-table", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the loss and the parameters after the last step of the headline timed window as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "train"):
+        ap.error("--dump-outputs writes the outputs of the GPU train step (--impl ours --workload train)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.impl == "reference":
         run_reference(args)
