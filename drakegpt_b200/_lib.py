@@ -15,7 +15,7 @@ MAJOR_K, MAJOR_MN = 0, 1
 
 EXPORTS = [
     "dgpt_last_error", "dgpt_abi_version", "dgpt_device_check", "dgpt_sm_count", "dgpt_debug_clock_probe", "dgpt_debug_clock_stamps",
-    "dgpt_dropout_keep_host", "dgpt_gemm_set_cta_group", "dgpt_dropout_scale", "dgpt_cast_bf16", "dgpt_embed_fwd",
+    "dgpt_dropout_keep_host", "dgpt_dropout_scale", "dgpt_cast_bf16", "dgpt_embed_fwd",
     "dgpt_embed_bwd", "dgpt_embed_ln_fwd", "dgpt_ln_fwd", "dgpt_ln_bwd", "dgpt_gemm", "dgpt_colsum", "dgpt_attn_fwd",
     "dgpt_attn_bwd", "dgpt_attn_bwd_scratch_bytes", "dgpt_cross_entropy", "dgpt_lmhead_ce", "dgpt_lmhead_ce_supported", "dgpt_gemm_res_ln", "dgpt_gemm_res_ln_supported", "dgpt_adamw", "dgpt_counter_add", "dgpt_sample",
     "dgpt_ipc_export", "dgpt_ipc_open", "dgpt_ipc_close", "dgpt_peer_copy", "dgpt_dp_adamw",
@@ -72,8 +72,6 @@ def _declare(lib):
     lib.dgpt_debug_clock_probe.argtypes = [C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
     lib.dgpt_debug_clock_stamps.restype = i32
     lib.dgpt_debug_clock_stamps.argtypes = [C.POINTER(C.c_uint64)]
-    lib.dgpt_gemm_set_cta_group.restype = i32
-    lib.dgpt_gemm_set_cta_group.argtypes = [i32]
     lib.dgpt_dropout_keep_host.restype = i32
     lib.dgpt_dropout_keep_host.argtypes = [u64, u32, u64, f32]
     sig = {

@@ -28,8 +28,9 @@ def _digest():
 
 
 def build(force=False, verbose=False, extra_flags=(), suffix=""):
-    """Build csrc/libdrakegpt_b200<suffix>.so.  ``extra_flags`` / ``suffix`` make experiment variants (e.g.
-    ``-DDGPT_STAGING_BUFS=1``) that are selected at run time with the DGPT_LIB environment variable."""
+    """Build csrc/libdrakegpt_b200<suffix>.so.  ``extra_flags`` / ``suffix`` make diagnostic variants (e.g.
+    ``-DDGPT_ATTN_TS``, the attention backward's phase stamps) that are selected at run time with the DGPT_LIB
+    environment variable."""
     lib = LIB.replace(".so", suffix + ".so")
     stamp = lib + ".stamp"
     dig = _digest() + " ".join(extra_flags)

@@ -12,21 +12,11 @@ int launch_attn_bwd_simt(const dgpt_attn_args* a, cudaStream_t st);
 int launch_attn_fwd_tc(const dgpt_attn_args* a, cudaStream_t st);
 int launch_attn_bwd_tc(const dgpt_attn_args* a, cudaStream_t st);
 bool attn_tc_supported(const dgpt_attn_args* a);
-void set_gemm_cta_group(int g);
 }  // namespace dgpt
 
 using namespace dgpt;
 
 extern "C" {
-
-int dgpt_gemm_set_cta_group(int cta_group) {
-  if (cta_group != 1 && cta_group != 2) {
-    set_error("gemm_set_cta_group: %d (must be 1 or 2)", cta_group);
-    return DGPT_E_ARG;
-  }
-  set_gemm_cta_group(cta_group);
-  return DGPT_OK;
-}
 
 int dgpt_gemm(const dgpt_gemm_args* a, void* stream) {
   DGPT_DEVICE_OR_RETURN();

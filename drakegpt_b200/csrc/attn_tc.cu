@@ -1,12 +1,13 @@
 // Tensor-mode fused causal attention for sm_100a (head size 64, T in {128, 256}).
 //
-// Forward  (one CTA per (batch, head, 128-query tile), two CTAs resident per SM):
+// Forward  (persistent: one CTA per SM walks a balanced list of (batch, head, 128-query tile)
+//   items, two in flight):
 //   TMA loads Q, K, V tiles (128B swizzle) -> tcgen05.mma S = Q K^T into TMEM (the whole
-//   128 x T score row block fits: no online rescaling) -> 128 softmax threads, one per
-//   query row, read S with tcgen05.ld, apply the causal mask, exp2, counter-based dropout, and
-//   write bf16 P back into TMEM (tcgen05.st, over the S columns already consumed) ->
+//   128 x T score row block fits: no online rescaling) -> one softmax thread per query row
+//   reads S with tcgen05.ld, applies the causal mask, exp2, counter-based dropout, and
+//   writes bf16 P back into TMEM (tcgen05.st, over the S columns already consumed) ->
 //   tcgen05.mma O = P V with P as the TMEM A operand and V consumed MN-major from its
-//   row-major shared-memory tile -> the same threads scale by 1/rowsum and store bf16 O at
+//   row-major shared-memory tile -> the same thread scales by 1/rowsum and stores bf16 O at
 //   column h*64 (the head concat is free).
 //   The T x T probabilities never touch HBM; only the log-sum-exp per row is saved.
 //
@@ -16,7 +17,6 @@
 //   MMAs accumulate dV += Pd^T dO, dK += dS^T Q, dQ += dS K in TMEM.  Every operand view
 //   (K-major or MN-major, transposed or not) is a descriptor over the same row-major tiles.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "ptx.cuh"
@@ -64,212 +64,7 @@ __device__ __forceinline__ void store_row32_sw128(uint8_t* tile_base, int row, i
 }
 
 // ===========================================================================
-// forward
-// ===========================================================================
-#ifdef DGPT_ATTN_TS
-__device__ long long g_attn_ts[64];
-#define ATS(i) do { if (blockIdx.x == 0 && blockIdx.y == 0 && blockIdx.z == (gridDim.z / 2) && lane == 0) g_attn_ts[i] = clock64(); } while (0)
-#else
-#define ATS(i) do { } while (0)
-#endif
-static constexpr int kFwdThreads = 192;
-static constexpr int kFwdSmem = 48 * 1024 + 32 * 1024 + 1024 + 128;  // Q, K (two tiles), V; P lives in TMEM
-
-__global__ void __launch_bounds__(kFwdThreads, 2)
-attn_fwd_tc_kernel(const __grid_constant__ CUtensorMap map_q, const __grid_constant__ CUtensorMap map_k,
-                   const __grid_constant__ CUtensorMap map_v, AttnTcP p) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint8_t* sQ = smem;                 // 16 KB
-  uint8_t* sK = smem + 16384;         // 2 x 16 KB
-  uint8_t* sV = smem + 49152;         // 4 x 8 KB (64 kv rows each)
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + 81920);
-  uint64_t *qk_full = bars, *v_full = bars + 1, *s_full = bars + 2, *p_full = bars + 3, *o_full = bars + 4;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 5);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (warp == 2) ATS(0);
-  const int ntile = p.T / QT;
-  const int qt = ntile - 1 - (int)blockIdx.x;  // heavier tiles first
-  const int h = blockIdx.y, b = blockIdx.z;
-  const int nkv = qt + 1;                      // key tiles this query tile can see
-  const int row0 = b * p.T;
-
-  if (threadIdx.x == 0) {
-    prefetch_tensormap(&map_q);
-    prefetch_tensormap(&map_k);
-    prefetch_tensormap(&map_v);
-    mbar_init(qk_full, 1);
-    mbar_init(v_full, 1);
-    mbar_init(s_full, 1);
-    mbar_init(p_full, 4);
-    mbar_init(o_full, 1);
-    fence_barrier_init();
-  }
-  if (warp == 1) tmem_alloc<256>(tmem_slot);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  pdl_grid_sync();  // prologue done (shared memory / TMEM only); global memory from here on
-  if (warp == 2) ATS(1);
-
-  if (warp == 0) {
-    if (elect_one()) {
-      mbar_expect_tx(qk_full, 16384 * (1 + nkv));
-      tma_load_2d(sQ, &map_q, qk_full, h * HD, row0 + qt * QT);
-      for (int j = 0; j < nkv; ++j) tma_load_2d(sK + j * 16384, &map_k, qk_full, h * HD, row0 + j * QT);
-      mbar_expect_tx(v_full, 8192 * 2 * nkv);
-      for (int kb = 0; kb < 2 * nkv; ++kb) tma_load_2d(sV + kb * 8192, &map_v, v_full, h * HD, row0 + kb * 64);
-    }
-  } else if (warp == 1) {
-    // the whole warp walks the (uniform) control flow, one elected lane issues: descriptors stay in uniform
-    // registers (an `if (lane == 0)` region makes the compiler wrap every MMA in an R2UR waterfall loop)
-    constexpr uint32_t idesc_s = make_idesc_bf16(128, 128, 0, 0);
-    constexpr uint32_t idesc_o = make_idesc_bf16(128, 64, 0, 1);
-    mbar_wait(qk_full, 0);
-    ATS(8);
-    tc_fence_after();
-    const uint64_t dq0 = make_smem_desc_sw128(smem_u32(sQ), 16, 1024);
-    const uint64_t dk0 = make_smem_desc_sw128(smem_u32(sK), 16, 1024);
-    if (elect_one()) {
-      for (int j = 0; j < nkv; ++j) {
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-          tc_mma_bf16(tmem + j * 128, dq0 + (uint64_t)(k * 2), dk0 + (uint64_t)(j * 1024 + k * 2), idesc_s, k > 0);
-      }
-      tc_commit(s_full);
-    }
-    __syncwarp();
-    mbar_wait(v_full, 0);
-    mbar_wait(p_full, 0);
-    tc_fence_after();
-    // O = P V with P read from TMEM (bf16 pairs, 8 columns per UMMA_K step; it overlays the consumed S columns)
-    // and V from shared memory (MN-major); O accumulates in the columns right above P
-    const uint64_t dv0 = make_smem_desc_sw128(smem_u32(sV), 8192, 1024);
-    if (elect_one()) {
-      for (int kb = 0; kb < 2 * nkv; ++kb) {
-#pragma unroll
-        for (int k = 0; k < 4; ++k)
-          tc_mma_bf16_ts(tmem + nkv * 64, tmem + kb * 32 + k * 8, dv0 + (uint64_t)(kb * 512 + k * 128), idesc_o, (kb | k) > 0);
-      }
-      tc_commit(o_full);
-    }
-    __syncwarp();
-  } else {
-    // ---------------------------- softmax + epilogue: one thread per query row ----------
-    const int quad = warp & 3;
-    const int row = quad * 32 + lane;
-    const int qg = qt * QT + row;  // query position inside the sequence
-    const uint32_t taddr = tmem + ((uint32_t)(quad * 32) << 16);
-    const int ncols = nkv * QT;
-    uint64_t seed = p.seed;
-    if (p.thr && p.seed_dev) seed += *p.seed_dev;
-    mbar_wait(s_full, 0);
-    if (warp == 2) ATS(2);
-    tc_fence_after();
-    // tcgen05.ld is warp-collective: loop bounds must be warp-uniform, so use the LAST row of this
-    // warp to decide which 32-column chunks are fully masked
-    const int qg_max = qt * QT + quad * 32 + 31;
-    // chunks entirely left of the diagonal for every row of this warp need no per-element causal test
-    const int qg_min = qt * QT + quad * 32;
-    float mx = -INFINITY;
-    for (int c = 0; c < ncols && c <= qg_max; c += 32) {
-      uint32_t r[32];
-      tmem_ld32(taddr + c, r);
-      tmem_ld_wait();
-      if (c + 31 <= qg_min) {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) mx = fmaxf(mx, __uint_as_float(r[j]));
-      } else {
-#pragma unroll
-        for (int j = 0; j < 32; ++j)
-          if (c + j <= qg) mx = fmaxf(mx, __uint_as_float(r[j]));
-      }
-    }
-    if (warp == 2) ATS(3);
-    const float sc = p.scale * kLog2e;
-    const float msc = mx * sc;
-    float sum = 0.f;
-    const uint64_t base = (((uint64_t)b * p.NH + h) * p.T + qg) * (uint64_t)p.T;
-    for (int c = 0; c < ncols; c += 32) {
-      float e[32];
-      if (c > qg_max) {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) e[j] = 0.f;
-      } else {
-        uint32_t r[32];
-        tmem_ld32(taddr + c, r);
-        tmem_ld_wait();
-        if (c + 31 <= qg_min) {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            const float v = exp2f(__uint_as_float(r[j]) * sc - msc);
-            sum += v;
-            e[j] = v;
-          }
-        } else {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            const float v = (c + j <= qg) ? exp2f(__uint_as_float(r[j]) * sc - msc) : 0.f;
-            sum += v;
-            e[j] = v;
-          }
-        }
-        if (p.thr) {  // the 32 keys of this chunk are one mask group (T % 32 == 0)
-          const DropGroup g = dropout_group(seed, p.site, (base + c) >> 5);
-#pragma unroll
-          for (int j = 0; j < 32; ++j)
-            if (dropout_word(g, j) < p.thr) e[j] = 0.f;
-        }
-      }
-      // bf16 P, two keys per 32-bit TMEM column, written over S columns [c / 2, c / 2 + 16): this thread has
-      // already consumed them (chunks <= c of its own row)
-      uint32_t pk[16];
-#pragma unroll
-      for (int j = 0; j < 16; ++j) pk[j] = pack_bf16(e[2 * j], e[2 * j + 1]);
-      tmem_st16(taddr + (c >> 1), pk);
-    }
-    if (p.lse) p.lse[((int64_t)b * p.NH + h) * p.T + qg] = mx * p.scale + logf(sum);
-    tmem_st_wait();
-    tc_fence_before();
-    __syncwarp();
-    if (lane == 0) mbar_arrive(p_full);
-    if (warp == 2) ATS(4);
-    // epilogue
-    mbar_wait(o_full, 0);
-    if (warp == 2) ATS(5);
-    tc_fence_after();
-    const float oscale = p.inv_keep / sum;
-    __nv_bfloat16* orow = reinterpret_cast<__nv_bfloat16*>(p.o) + (int64_t)(row0 + qg) * p.o_rs + h * HD;
-#pragma unroll
-    for (int c = 0; c < HD; c += 32) {
-      uint32_t r[32];
-      tmem_ld32(taddr + nkv * 64 + c, r);
-      tmem_ld_wait();
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        uint4 w;
-        w.x = pack_bf16(__uint_as_float(r[8 * j]) * oscale, __uint_as_float(r[8 * j + 1]) * oscale);
-        w.y = pack_bf16(__uint_as_float(r[8 * j + 2]) * oscale, __uint_as_float(r[8 * j + 3]) * oscale);
-        w.z = pack_bf16(__uint_as_float(r[8 * j + 4]) * oscale, __uint_as_float(r[8 * j + 5]) * oscale);
-        w.w = pack_bf16(__uint_as_float(r[8 * j + 6]) * oscale, __uint_as_float(r[8 * j + 7]) * oscale);
-        *reinterpret_cast<uint4*>(orow + c + 8 * j) = w;
-      }
-    }
-  }
-  if (warp == 2) ATS(6);
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tc_fence_after();
-    tmem_dealloc<256>(tmem);
-  }
-  if (warp == 2) ATS(7);
-}
-
-// ===========================================================================
-// forward, persistent form (DGPT_ATTN_FWD=2, the default): one CTA per SM walks a statically balanced list of (batch, head, query
+// forward, persistent: one CTA per SM walks a statically balanced list of (batch, head, query
 // tile) items with TWO items in flight, so that the serial phases of one item (TMA latency, S MMAs, softmax, P V,
 // output) are filled with the other item's work instead of idling the SM:
 //   warp 8   TMA producer: Q / K and V tiles of item n into stage n & 1 (the Q / K stage is released as soon as the
@@ -563,295 +358,11 @@ attn_fwd_tc2_kernel(const __grid_constant__ CUtensorMap map_q32, const __grid_co
 }
 
 // ===========================================================================
-// forward, persistent form with TWO softmax threads per query row (DGPT_ATTN_FWD=3; measured slower with dropout).  Same pipeline as attn_fwd_tc2_kernel
-// (two items in flight, TMA producer and tcgen05 issuer on the highest warp ids), but a warpgroup is 8 warps: thread A
-// of a row (warps 0-3 of the group) owns the first half of the key columns, thread B (warps 4-7, same TMEM lane
-// quadrant) the second half, so the serial exp2 / dropout / pack chain of an item is half as long and 16 softmax
-// warps instead of 8 hide each other's latencies.  Row max and row sum are exchanged through shared memory (two
-// named barriers per item).  P (bf16) of each half overlays the S columns its own thread has consumed:
-//     keys [0, n/2) -> columns [0, n/4),  keys [n/2, n) -> columns [n/2, 3n/4);  O above both (n = 128 or 256 keys).
-// ===========================================================================
-static constexpr int kFwd3Threads = 576;  // 16 softmax warps, TMA producer (warp 16), tcgen05 issuer (warp 17)
-static constexpr int kFwd3Smem = 2 * kFwd2QK + 2 * 32768 + 4096 + 256 + 1024;
-
-__global__ void __launch_bounds__(kFwd3Threads, 1)
-attn_fwd_tc3_kernel(const __grid_constant__ CUtensorMap map_q32, const __grid_constant__ CUtensorMap map_k,
-                    const __grid_constant__ CUtensorMap map_v, AttnTcP p, FwdSched sc) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
-  uint8_t* sQK = smem;                    // [2][Q | K0 | K1]
-  uint8_t* sV = smem + 2 * kFwd2QK;       // [2][4 x 8 KB]
-  float* xch = reinterpret_cast<float*>(sV + 2 * 32768);  // [2 groups][max: 2 x 128 | sum: 2 x 128]
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sV + 2 * 32768 + 4096);
-  uint64_t *qk_full = bars, *qk_empty = bars + 2, *v_full = bars + 4, *v_empty = bars + 6, *s_full = bars + 8,
-           *p_full = bars + 10, *o_full = bars + 12, *slot_free = bars + 14;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 16);
-
-  clock_probe_begin(sc.probe);
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int ntile = p.T / QT;
-
-  // ---- this CTA's item list (see attn_fwd_tc2_kernel) ----
-  const int G = gridDim.x, c = blockIdx.x;
-  const int hq = sc.nheavy / G, hr = sc.nheavy % G;
-  const int nh_c = hq + (c < hr ? 1 : 0);
-  const int U = (kWHeavy * sc.nheavy + kWLight * sc.nlight + G - 1) / G;
-  const int cap_hi = max(0, (U - kWHeavy * (hq + 1)) / kWLight), cap_lo = max(0, (U - kWHeavy * hq) / kWLight);
-  const int cap_total = hr * cap_hi + (G - hr) * cap_lo;
-  const int l_start = c < hr ? c * cap_hi : hr * cap_hi + (c - hr) * cap_lo;
-  const int l0 = min(sc.nlight, l_start), l1 = min(sc.nlight, l_start + (c < hr ? cap_hi : cap_lo));
-  const int n_extra = cap_total < sc.nlight ? (sc.nlight - cap_total - c + G - 1) / G : 0;
-  const int n_items = nh_c + (l1 - l0) + max(0, n_extra);
-  auto item = [&](int n, int& bh, int& qt) {
-    if (n < nh_c) {
-      bh = c + n * G; qt = ntile - 1;
-    } else {
-      const int m = n - nh_c;
-      bh = m < l1 - l0 ? l0 + m : cap_total + c + (m - (l1 - l0)) * G;
-      qt = 0;
-    }
-  };
-
-  if (threadIdx.x == 0) {
-    prefetch_tensormap(&map_q32);
-    prefetch_tensormap(&map_k);
-    prefetch_tensormap(&map_v);
-    for (int g = 0; g < 2; ++g) {
-      mbar_init(&qk_full[g], 1);
-      mbar_init(&qk_empty[g], 1);
-      mbar_init(&v_full[g], 1);
-      mbar_init(&v_empty[g], 1);
-      mbar_init(&s_full[g], 1);
-      mbar_init(&p_full[g], 8);
-      mbar_init(&o_full[g], 1);
-      mbar_init(&slot_free[g], 8);
-    }
-    fence_barrier_init();
-  }
-  if (warp == 17) tmem_alloc<512>(tmem_slot);
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem = *tmem_slot;
-  pdl_grid_sync();  // prologue done (shared memory / TMEM only); global memory from here on
-
-  if (warp == 16) {
-    // ------------------------------ TMA producer ---------------------------
-    for (int n = 0; n < n_items; ++n) {
-      const int g = n & 1, k = n >> 1;
-      int bh, qt;
-      item(n, bh, qt);
-      const int nkv = qt + 1, b = bh / p.NH, h = bh % p.NH, row0 = b * p.T;
-      uint8_t* q_s = sQK + g * kFwd2QK;
-      uint8_t* v_s = sV + g * 32768;
-      mbar_wait(&qk_empty[g], (k & 1) ^ 1);
-      if (elect_one()) {
-        mbar_expect_tx(&qk_full[g], 16384 * (1 + nkv));
-        for (int qb = 0; qb < 4; ++qb)  // group 1 takes its query row blocks in reverse order (sub-partition balance)
-          tma_load_2d(q_s + qb * 4096, &map_q32, &qk_full[g], h * HD, row0 + qt * QT + (g ? 3 - qb : qb) * 32);
-        for (int j = 0; j < nkv; ++j) tma_load_2d(q_s + 16384 * (1 + j), &map_k, &qk_full[g], h * HD, row0 + j * QT);
-      }
-      __syncwarp();
-      mbar_wait(&v_empty[g], (k & 1) ^ 1);
-      if (elect_one()) {
-        mbar_expect_tx(&v_full[g], 16384 * nkv);
-        for (int kb = 0; kb < 2 * nkv; ++kb) tma_load_2d(v_s + kb * 8192, &map_v, &v_full[g], h * HD, row0 + kb * 64);
-      }
-      __syncwarp();
-    }
-  } else if (warp == 17) {
-    // ------------------------------ MMA issuer -----------------------------
-    constexpr uint32_t idesc_s = make_idesc_bf16(128, 128, 0, 0);
-    constexpr uint32_t idesc_o = make_idesc_bf16(128, 64, 0, 1);
-    int next_s = 0, next_pv = 0;
-    while (next_pv < n_items) {
-      bool progressed = false;
-      if (next_s < n_items) {
-        const int g = next_s & 1, k = next_s >> 1;
-        if (mbar_test(&qk_full[g], k & 1) && mbar_test(&slot_free[g], (k & 1) ^ 1)) {
-          tc_fence_after();
-          int bh, qt;
-          item(next_s, bh, qt);
-          const int nkv = qt + 1;
-          const uint64_t dq0 = make_smem_desc_sw128(smem_u32(sQK + g * kFwd2QK), 16, 1024);
-          const uint64_t dk0 = make_smem_desc_sw128(smem_u32(sQK + g * kFwd2QK + 16384), 16, 1024);
-          if (elect_one()) {
-            for (int j = 0; j < nkv; ++j) {
-#pragma unroll
-              for (int kk = 0; kk < 4; ++kk)
-                tc_mma_bf16(tmem + g * 256 + j * 128, dq0 + (uint64_t)(kk * 2), dk0 + (uint64_t)(j * 1024 + kk * 2), idesc_s, kk > 0);
-            }
-            tc_commit(&s_full[g]);
-            tc_commit(&qk_empty[g]);
-          }
-          __syncwarp();
-          ++next_s;
-          progressed = true;
-        }
-      }
-      if (next_pv < next_s) {
-        const int g = next_pv & 1, k = next_pv >> 1;
-        if (mbar_test(&p_full[g], k & 1) && mbar_test(&v_full[g], k & 1)) {
-          tc_fence_after();
-          int bh, qt;
-          item(next_pv, bh, qt);
-          const int nkv = qt + 1;
-          const uint32_t ocol = nkv == 2 ? 192u : 128u;
-          const uint64_t dv0 = make_smem_desc_sw128(smem_u32(sV + g * 32768), 8192, 1024);
-          if (elect_one()) {
-            for (int kb = 0; kb < 2 * nkv; ++kb) {
-              // P of the 64-key block kb: first half of the keys at columns [0, ..), second half at [nkv * 64, ..)
-              const uint32_t pcol = kb < nkv ? (uint32_t)(kb * 32) : (uint32_t)(nkv * 64 + (kb - nkv) * 32);
-#pragma unroll
-              for (int kk = 0; kk < 4; ++kk)
-                tc_mma_bf16_ts(tmem + g * 256 + ocol, tmem + g * 256 + pcol + kk * 8, dv0 + (uint64_t)(kb * 512 + kk * 128), idesc_o,
-                               (kb | kk) > 0);
-            }
-            tc_commit(&o_full[g]);
-            tc_commit(&v_empty[g]);
-          }
-          __syncwarp();
-          ++next_pv;
-          progressed = true;
-        }
-      }
-      if (!progressed) __nanosleep(32);
-    }
-  } else {
-    // ---------------------------- softmax + output: two threads per query row ----------
-    const int g = warp >> 3;            // warpgroup = TMEM slot = shared-memory stage
-    const int quad = warp & 3;
-    const int hc = (warp >> 2) & 1;     // 0: first half of the key columns, 1: second half
-    const int rblk = g ? 3 - quad : quad;
-    const int row = rblk * 32 + lane;
-    const uint32_t taddr = tmem + (uint32_t)(g * 256) + ((uint32_t)(quad * 32) << 16);
-    float* xmax = xch + g * 512;        // [2][128]
-    float* xsum = xmax + 256;           // [2][128]
-    uint64_t seed = p.seed;
-    if (p.thr && p.seed_dev) seed += *p.seed_dev;
-    const float sc2 = p.scale * kLog2e;
-    for (int n = g; n < n_items; n += 2) {
-      const int k = n >> 1;
-      int bh, qt;
-      item(n, bh, qt);
-      const int nkv = qt + 1, b = bh / p.NH, h = bh % p.NH, row0 = b * p.T;
-      const int qg = qt * QT + row;             // query position inside the sequence
-      const int hcols = nkv * (QT / 2);         // key columns per thread: 64 or 128
-      const int c_beg = hc * hcols, c_end = c_beg + hcols;
-      const uint32_t pbase = hc ? (uint32_t)hcols : 0u;  // where this thread's P goes (32-bit TMEM columns)
-      const uint32_t ocol = nkv == 2 ? 192u : 128u;
-#define FTS3(i) do { if (sc.probe && blockIdx.x == 0 && warp == 0 && lane == 0 && k < 3) sc.probe[4 + k * 8 + (i)] = (unsigned long long)clock64(); } while (0)
-      FTS3(0);
-      mbar_wait(&s_full[g], k & 1);
-      FTS3(1);
-      tc_fence_after();
-      const int qg_max = qt * QT + rblk * 32 + 31, qg_min = qt * QT + rblk * 32;  // (warp-uniform loop bounds)
-      float mx = -INFINITY;
-      for (int cc = c_beg; cc < c_end && cc <= qg_max; cc += 32) {
-        uint32_t r[32];
-        tmem_ld32(taddr + cc, r);
-        tmem_ld_wait();
-        if (cc + 31 <= qg_min) {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) mx = fmaxf(mx, __uint_as_float(r[j]));
-        } else {
-#pragma unroll
-          for (int j = 0; j < 32; ++j)
-            if (cc + j <= qg) mx = fmaxf(mx, __uint_as_float(r[j]));
-        }
-      }
-      xmax[hc * 128 + quad * 32 + lane] = mx;
-      asm volatile("bar.sync %0, 256;" ::"r"(2 + g) : "memory");
-      mx = fmaxf(mx, xmax[(hc ^ 1) * 128 + quad * 32 + lane]);  // (the first half always holds key 0: finite)
-      FTS3(2);
-      const float msc = mx * sc2;
-      float sum = 0.f;
-      const uint64_t base = (((uint64_t)b * p.NH + h) * p.T + qg) * (uint64_t)p.T;
-      DropGroup dg = {0u, 0u};
-      for (int cc = c_beg; cc < c_end; cc += 16) {
-        float e[16];
-        if (cc > qg_max) {
-#pragma unroll
-          for (int j = 0; j < 16; ++j) e[j] = 0.f;
-        } else {
-          uint32_t r[16];
-          tmem_ld16(taddr + cc, r);
-          tmem_ld_wait();
-          if (cc + 15 <= qg_min) {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) {
-              const float v = exp2f(__uint_as_float(r[j]) * sc2 - msc);
-              sum += v;
-              e[j] = v;
-            }
-          } else {
-#pragma unroll
-            for (int j = 0; j < 16; ++j) {
-              const float v = (cc + j <= qg) ? exp2f(__uint_as_float(r[j]) * sc2 - msc) : 0.f;
-              sum += v;
-              e[j] = v;
-            }
-          }
-          if (p.thr) {  // 32 keys are one mask group (T % 32 == 0): one hash per two 16-key steps
-            if ((cc & 16) == 0) dg = dropout_group(seed, p.site, (base + cc) >> 5);
-            const uint32_t e0 = (uint32_t)(cc & 16);
-#pragma unroll
-            for (int j = 0; j < 16; ++j)
-              if (dropout_word(dg, e0 + j) < p.thr) e[j] = 0.f;
-          }
-        }
-        uint32_t pk[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) pk[j] = pack_bf16(e[2 * j], e[2 * j + 1]);
-        tmem_st8(taddr + pbase + (uint32_t)((cc - c_beg) >> 1), pk);
-      }
-      xsum[hc * 128 + quad * 32 + lane] = sum;
-      tmem_st_wait();
-      tc_fence_before();
-      asm volatile("bar.sync %0, 256;" ::"r"(2 + g) : "memory");
-      sum += xsum[(hc ^ 1) * 128 + quad * 32 + lane];
-      if (hc == 0 && p.lse) p.lse[((int64_t)b * p.NH + h) * p.T + qg] = mx * p.scale + logf(sum);
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&p_full[g]);
-      FTS3(3);
-      // output: each of the two threads of a row converts and stores half of the 64 head dims
-      mbar_wait(&o_full[g], k & 1);
-      FTS3(4);
-      tc_fence_after();
-      const float oscale = p.inv_keep / sum;
-      __nv_bfloat16* orow = reinterpret_cast<__nv_bfloat16*>(p.o) + (int64_t)(row0 + qg) * p.o_rs + h * HD + hc * 32;
-      {
-        uint32_t r[32];
-        tmem_ld32(taddr + ocol + hc * 32, r);
-        tmem_ld_wait();
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-          uint4 w;
-          w.x = pack_bf16(__uint_as_float(r[8 * j]) * oscale, __uint_as_float(r[8 * j + 1]) * oscale);
-          w.y = pack_bf16(__uint_as_float(r[8 * j + 2]) * oscale, __uint_as_float(r[8 * j + 3]) * oscale);
-          w.z = pack_bf16(__uint_as_float(r[8 * j + 4]) * oscale, __uint_as_float(r[8 * j + 5]) * oscale);
-          w.w = pack_bf16(__uint_as_float(r[8 * j + 6]) * oscale, __uint_as_float(r[8 * j + 7]) * oscale);
-          *reinterpret_cast<uint4*>(orow + 8 * j) = w;
-        }
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&slot_free[g]);  // TMEM slot g may take the S of item n + 2
-      FTS3(5);
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 17) {
-    tc_fence_after();
-    tmem_dealloc<512>(tmem);
-  }
-  clock_probe_end(sc.probe);
-}
-
-// ===========================================================================
 // backward
 // ===========================================================================
+#ifdef DGPT_ATTN_TS
+__device__ long long g_attn_ts[64];  // phase stamps of one CTA (BTS below), printed by launch_attn_bwd_tc
+#endif
 static constexpr int kBwdThreads = 64 + 256;
 static constexpr int kBwdSmem = 8 * 16384 + 2 * 32768 + 16384 + 2048 + 1024 + 128;
 
@@ -1225,71 +736,30 @@ static AttnTcP make_tc_params(const dgpt_attn_args* a) {
   return p;
 }
 
-// DGPT_ATTN_FWD: 1 = the round-1 one-item-per-CTA kernel (26.6 us at the model shape), 2 = persistent, one softmax
-// thread per row (default: 23.2 us with dropout 0.2, 21.3 without), 3 = persistent, two softmax threads per row
-// (20.8 us without dropout but 28.5 us with it: 16 softmax warps saturate the issue slots the mask costs)
-static int attn_fwd_variant() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("DGPT_ATTN_FWD"); v = e ? atoi(e) : 2; }
-  return v;
-}
-
 int launch_attn_fwd_tc(const dgpt_attn_args* a, cudaStream_t st) {
   CUtensorMap mq, mk, mv;
   const int64_t rows = (int64_t)a->B * a->Tk, cols = (int64_t)a->NH * HD;
   int rc;
-  if ((rc = make_tmap_bf16_2d(&mq, a->q, cols, rows, a->q_rs, QT))) return rc;
+  if ((rc = make_tmap_bf16_2d(&mq, a->q, cols, rows, a->q_rs, 32))) return rc;  // 32-row blocks (see the producer)
   if ((rc = make_tmap_bf16_2d(&mk, a->k, cols, rows, a->k_rs, QT))) return rc;
   if ((rc = make_tmap_bf16_2d(&mv, a->v, cols, rows, a->v_rs, 64))) return rc;
   AttnTcP p = make_tc_params(a);
-  if (attn_fwd_variant() != 1) {
-    if ((rc = make_tmap_bf16_2d(&mq, a->q, cols, rows, a->q_rs, 32))) return rc;  // 32-row blocks (see the producer)
-    static bool attr2 = false;
-    if (!attr2) {
-      cudaError_t e = cudaFuncSetAttribute(attn_fwd_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwd2Smem);
-      if (e != cudaSuccess) { set_error("attn_fwd_tc2: smem attribute: %s", cudaGetErrorString(e)); return DGPT_E_LAUNCH; }
-      attr2 = true;
-    }
-    const int ntile = a->Tk / QT, bh = a->B * a->NH;
-    FwdSched sc;
-    sc.nheavy = ntile > 1 ? bh : 0;
-    sc.nlight = bh;
-    sc.probe = clock_probe_buffer();
-    int sms = dgpt_sm_count();
-    if (sms <= 0) sms = 148;
-    const int grid = min(sms, sc.nheavy + sc.nlight);
-    if (attn_fwd_variant() == 3) {
-      static bool attr3 = false;
-      if (!attr3) {
-        cudaError_t e = cudaFuncSetAttribute(attn_fwd_tc3_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwd3Smem);
-        if (e != cudaSuccess) { set_error("attn_fwd_tc3: smem attribute: %s", cudaGetErrorString(e)); return DGPT_E_LAUNCH; }
-        attr3 = true;
-      }
-      launch_pdl(attn_fwd_tc3_kernel, dim3(grid), dim3(kFwd3Threads), kFwd3Smem, st, mq, mk, mv, p, sc);
-      return check_launch("attn_fwd_tc3");
-    }
-    launch_pdl(attn_fwd_tc2_kernel, dim3(grid), dim3(kFwd2Threads), kFwd2Smem, st, mq, mk, mv, p, sc);
-    return check_launch("attn_fwd_tc2");
-  }
   static bool attr = false;
   if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(attn_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwdSmem);
-    if (e != cudaSuccess) { set_error("attn_fwd_tc: smem attribute: %s", cudaGetErrorString(e)); return DGPT_E_LAUNCH; }
+    cudaError_t e = cudaFuncSetAttribute(attn_fwd_tc2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kFwd2Smem);
+    if (e != cudaSuccess) { set_error("attn_fwd_tc2: smem attribute: %s", cudaGetErrorString(e)); return DGPT_E_LAUNCH; }
     attr = true;
   }
-  dim3 grid(a->Tk / QT, a->NH, a->B);
-  launch_pdl(attn_fwd_tc_kernel, grid, dim3(kFwdThreads), kFwdSmem, st, mq, mk, mv, p);
-#ifdef DGPT_ATTN_TS
-  {
-    cudaStreamSynchronize(st);
-    long long h[64];
-    cudaMemcpyFromSymbol(h, g_attn_ts, sizeof(h));
-    printf("attn fwd CTA(qt=1,h=0,b=B/2): setup %lld | qk load done %lld | S ready %lld | pass1 %lld | pass2 %lld | PV wait %lld | epilogue %lld | exit %lld\n",
-           h[1] - h[0], h[8] - h[0], h[2] - h[0], h[3] - h[2], h[4] - h[3], h[5] - h[4], h[6] - h[5], h[7] - h[6]);
-    fflush(stdout);
-  }
-#endif
-  return check_launch("attn_fwd_tc");
+  const int ntile = a->Tk / QT, bh = a->B * a->NH;
+  FwdSched sc;
+  sc.nheavy = ntile > 1 ? bh : 0;
+  sc.nlight = bh;
+  sc.probe = clock_probe_buffer();
+  int sms = dgpt_sm_count();
+  if (sms <= 0) sms = 148;
+  const int grid = min(sms, sc.nheavy + sc.nlight);
+  launch_pdl(attn_fwd_tc2_kernel, dim3(grid), dim3(kFwd2Threads), kFwd2Smem, st, mq, mk, mv, p, sc);
+  return check_launch("attn_fwd_tc2");
 }
 
 int launch_attn_bwd_tc(const dgpt_attn_args* a, cudaStream_t st) {

@@ -6,7 +6,9 @@
 // split-K / accumulate -- so the output is written in full 128-byte lines, clipped at the
 // matrix edge by the tensor map, with no per-thread global stores.  Persistent: one CTA
 // per SM walks the tile list; TMEM holds two accumulators so the epilogue of tile i
-// overlaps the mainloop of tile i+1.
+// overlaps the mainloop of tile i+1.  Long-K GEMMs of the big activations use 256-row
+// CTA tiles (two M = 128 MMAs per k-step on one B stage, see TcCfg), and wgrads can
+// carry the bias gradient as a column-sum MMA.
 //
 // Warp roles (320 threads): warp 0 = TMA producer, warp 1 = TMEM owner + MMA
 // issuer, warps 2..9 = epilogue (TMEM lane quadrant = warp_id % 4, two warps per quadrant).
@@ -16,7 +18,6 @@
 // dgrad / wgrad need) are both fed straight from the row-major tensors -- no
 // transposed copies are ever written to HBM.
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "epilogue.cuh"
 #include "ptx.cuh"
@@ -38,12 +39,6 @@ struct TcParams {
   int m_tiles, n_tiles, split_k, kb_total, kb_per_split;
   int vec_ok;      // epilogue operands (bias / residual) allow the vector fast path
   int store_mode;  // StoreMode for D
-  int cta_group;   // 1, or 2 = CTA pairs (cluster of 2) sharing each MMA
-  int coalesced;   // output blocks leave by coalesced st.global from the staging tile instead of TMA stores
-  int role_hi;     // warp-role placement: 1 = producer / MMA issuer take the two HIGHEST warp ids (8, 9)
-  int debug;       // DGPT_GEMM_DEBUG bits (timing experiments only): 1 = epilogue skipped, 2 = no TMA loads / MMAs,
-                   // 4 = epilogue without the output stores, 8 = epilogue without the math, 16 / 32 = B operand loaded on
-                   // every other k-block / never (port-traffic experiments)
   unsigned long long* probe; // DGPT_CLOCK_PROBE stamps (or NULL)
   uint32_t* mask_out;        // ReLU bit mask written by the forward GEMM  [(n / 32) * M + m]
   const uint32_t* mask_in;   // ... and applied by the dgrad GEMM
@@ -54,29 +49,24 @@ struct TcParams {
 // epilogue feature bits (compile-time mask of the fused epilogue, or -1 = generic element-wise path)
 enum { kEpiBias = 1, kEpiRelu = 2, kEpiAux = 4, kEpiDrop = 8, kEpiRes = 16, kEpiMaskIn = 32, kEpiMaskOut = 64 };
 
-// CG = CTAs sharing one MMA (tcgen05 cta_group).  With CG = 2 a pair of CTAs computes a 256 x BN tile: each CTA
-// stages its own 128 rows of A but only HALF of B (the MMA reads the other half from the peer's shared memory).
-// RESBUFS != 0: the fp32 residual operand arrives by TMA into the epilogue staging buffers, see the epilogue below.
-// 4 buffers per warp = the next tile's residual is fetched while this tile's stores drain (short-K GEMMs, whose
-// epilogue is the critical path; ring of 3 stages); 2 buffers = fetched once this tile's stores have been read
-// (long-K GEMMs: the epilogue warps have slack, the mainloop wants the 5-stage ring).
+// EPI: epilogue feature mask (see the kernel).  With kEpiRes the fp32 residual operand arrives by TMA into the
+// epilogue staging buffers, see the epilogue below: the next tile's residual is fetched once this tile's stores have
+// been read out of them.
 // TM = 128-row sub-tiles per CTA tile (1 or 2).  TM = 2: a 256 x BN tile as two M = 128 MMAs per k-step that share one
 // B stage -- 2/3 of the operand bytes per MMA cycle of a 128 x BN tile (measured: the mainloop of 128-row tiles waits
 // for operands 30-50 % of the time, the SM ingests ~70 B/cycle and a 128 x 256 tile needs 94).  The two accumulators
 // fill TMEM (2 x 256 or 2 x 192 columns), so TM = 2 tiles are single-buffered: the epilogue of a tile does not overlap
 // the mainloop of the next one, which costs little because such GEMMs are launched with <= ~3 tiles per CTA.
-template <int BN, int CG, int RESBUFS, int CS = 0, int TM = 1>
+template <int BN, int EPI, int CS = 0, int TM = 1>
 struct TcCfg {
+  static constexpr bool kRes = EPI >= 0 && (EPI & kEpiRes) != 0;
   static constexpr int kABytes = TM * TBM * TBK * 2;
-  static constexpr int kBBytes = (BN / CG) * TBK * 2;
+  static constexpr int kBBytes = BN * TBK * 2;
   static constexpr int kStageBytes = kABytes + kBBytes;
-  // 4 KB staging buffers per epilogue warp: 2, or (residual epilogues) the warp's fp32 blocks of one tile
-  // (RESBUFS = 2) or of two tiles (RESBUFS = 4); TM = 2 keeps one (the ring needs the room)
+  // 4 KB staging buffers per epilogue warp: 2, or (residual epilogues) one per fp32 block of the warp's half of a
+  // tile; TM = 2 keeps one (the ring needs the room)
   static constexpr int kResBlocks = BN / 2 / 32;
-#ifndef DGPT_STAGING_BUFS
-#define DGPT_STAGING_BUFS 2
-#endif
-  static constexpr int kStagingBufs = RESBUFS ? (RESBUFS / 2) * kResBlocks : (TM == 2 ? 1 : DGPT_STAGING_BUFS);
+  static constexpr int kStagingBufs = kRes ? kResBlocks : (TM == 2 ? 1 : 2);
   static constexpr int kStagingBytes = 8 * kStagingBufs * 4096;
   static constexpr int kBiasBytes = 2 * BN * 4;  // bias slice of the tile, double-buffered with the accumulator
   static constexpr int kBarBytes = 512;
@@ -87,7 +77,7 @@ struct TcCfg {
   static constexpr int kTmemNeed = kNAcc * TM * BN + (CS ? kNAcc * TM * 16 : 0);
   static constexpr int kTmemCols = kTmemNeed <= 32 ? 32 : kTmemNeed <= 64 ? 64 : kTmemNeed <= 128 ? 128 : kTmemNeed <= 256 ? 256 : 512;
   static_assert(kTmemNeed <= 512, "no TMEM room");
-  static_assert(TM == 1 || (CG == 1 && RESBUFS == 0), "256-row CTA tiles: single-CTA MMAs, no TMA-fed residual");
+  static_assert(TM == 1 || !kRes, "256-row CTA tiles: no TMA-fed residual");
   static constexpr size_t kSmemBytes = (size_t)kStages * kStageBytes + kStagingBytes + kBiasBytes + kBarBytes;
   static_assert(kStages >= 3, "shared-memory ring too shallow");
 };
@@ -214,25 +204,26 @@ __device__ __forceinline__ bool kb_nonempty(const TcParams& p, int ks) { return 
 // the kernel
 //   EPI  : compile-time epilogue feature mask (fast path), or -1 = generic element-wise epilogue
 //   OBF  : output element type of the fast path (1 = bf16, 0 = fp32); ignored when EPI < 0
+//   CS   : 1 = column sums, see below
+//   TM   : 128-row sub-tiles per CTA tile (see TcCfg)
 // --------------------------------------------------------------------------
-// CS = 1 (wgrad form: A MN-major, plain fp32 epilogue, CG = 1): the column sums of the stored A matrix
+// CS = 1 (wgrad form: A MN-major, plain fp32 epilogue): the column sums of the stored A matrix
 // (= row sums of the logical A: sum_k A[m, k], the bias gradient when A = dY^T) ride on the tensor core as
 // one extra N = 16 MMA per k-step against an all-ones B tile -- no separate pass over dY.
-template <int BN, int A_MN, int B_MN, int EPI, int OBF, int CG, int RESBUFS, int CS, int TM>
+template <int BN, int A_MN, int B_MN, int EPI, int OBF, int CS, int TM>
 __global__ void __launch_bounds__(kThreads, 1)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
                const __grid_constant__ CUtensorMap map_d, const __grid_constant__ CUtensorMap map_r, TcParams p) {
-  constexpr bool kRes = EPI >= 0 && (EPI & kEpiRes) != 0;
-  static_assert(kRes == (RESBUFS != 0), "RESBUFS goes with the residual epilogues");
-  using Cfg = TcCfg<BN, CG, RESBUFS, CS, TM>;
-  static_assert(!CS || (CG == 1 && EPI == 0), "column sums: single-CTA tiles, plain epilogue");
+  using Cfg = TcCfg<BN, EPI, CS, TM>;
+  constexpr bool kRes = Cfg::kRes;
+  static_assert(!CS || EPI == 0, "column sums: plain epilogue");
   constexpr int kStages = Cfg::kStages;
   constexpr int kABytes = Cfg::kABytes;
   constexpr int kNAcc = Cfg::kNAcc;
   constexpr int kTileM = TBM * TM;        // rows of a CTA tile
   constexpr int kAccCols = TM * BN;       // TMEM columns of one accumulator buffer
   constexpr int kBBytes = Cfg::kBBytes;
-  constexpr uint32_t kIdesc = make_idesc_bf16(TBM * CG, BN, A_MN, B_MN);
+  constexpr uint32_t kIdesc = make_idesc_bf16(TBM, BN, A_MN, B_MN);
 
   extern __shared__ __align__(1024) uint8_t smem[];  // SWIZZLE_128B tiles need 1024-byte alignment
   uint8_t* stage_base = smem;
@@ -242,17 +233,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   uint64_t* empty_bar = full_bar + 8;
   uint64_t* tmem_full = empty_bar + 8;
   uint64_t* tmem_empty = tmem_full + 2;
-  uint64_t* res_bar = tmem_empty + 2;  // [8 epilogue warps][2 tiles in flight]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(res_bar + 16);
+  uint64_t* res_bar = tmem_empty + 2;  // [8 epilogue warps]
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(res_bar + 8);
 
-  // Warp roles.  The issue arbiter of an SM sub-partition favours the HIGHEST warp id among its eligible warps
-  // (B300_MICROARCH: hi-wid-first), and a warp's sub-partition AND its TMEM lane quadrant are both warp_id % 4, so
-  // the MMA-issuing warp always shares its scheduler with two epilogue warps: with role_hi the producer and the
-  // issuer are warps 8 and 9 (they win the arbitration whenever they are eligible) and the epilogue is warps 0..7;
-  // `warp` below is the LOGICAL role id (0 producer, 1 issuer, 2..9 epilogue), `pwarp` the physical warp.
   clock_probe_begin(p.probe);
-  const int pwarp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int warp = p.role_hi ? (pwarp >= 8 ? pwarp - 8 : pwarp + 2) : pwarp;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
   if (threadIdx.x == 0) {
     prefetch_tensormap(&map_a);
@@ -265,9 +250,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     }
     for (int i = 0; i < 2; ++i) {
       mbar_init(&tmem_full[i], 1);
-      mbar_init(&tmem_empty[i], 8 * CG);  // one arrive per epilogue warp of every CTA sharing the accumulator
+      mbar_init(&tmem_empty[i], 8);  // one arrive per epilogue warp
     }
-    for (int i = 0; i < 16; ++i) mbar_init(&res_bar[i], 1);
+    for (int i = 0; i < 8; ++i) mbar_init(&res_bar[i], 1);
     fence_barrier_init();
   }
   if (CS && warp >= 2) {
@@ -276,17 +261,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     for (int i = (warp - 2) * 32 + lane; i < 256; i += 256) ones[i] = 0x3F803F80u;
     fence_proxy_async();  // generic-proxy writes -> visible to the MMA's async-proxy reads (after the barrier below)
   }
-  if (CG == 2) {  // both CTAs of the pair have initialised their barriers before the paired TMEM allocation
-    __syncthreads();
-    cluster_sync_all();
-  }
-  if (warp == 1) {
-    if (CG == 1) tmem_alloc<Cfg::kTmemCols>(tmem_slot);
-    else tmem_alloc_2sm<Cfg::kTmemCols>(tmem_slot);
-  }
+  if (warp == 1) tmem_alloc<Cfg::kTmemCols>(tmem_slot);
   tc_fence_before();
   __syncthreads();
-  if (CG == 2) cluster_sync_all();  // the peer's TMEM and barriers exist before anything is sent to them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
   // everything above touched only this CTA's shared memory / TMEM: with programmatic dependent launch it overlapped
@@ -294,12 +271,10 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
   pdl_launch_dependents();
   pdl_wait();
 
-  // tile walk: with CG = 2 the pair handles pair-tiles (256 rows) and CTA rank r takes rows [128 r, 128 r + 128)
   const bool prof = p.probe != nullptr && blockIdx.x == 0;  // DGPT_CLOCK_PROBE: where the roles of CTA 0 wait
-  const int crank = CG == 2 ? (int)cluster_ctarank() : 0;
-  const int tiles_mn = (p.m_tiles / CG) * p.n_tiles;
+  const int tiles_mn = p.m_tiles * p.n_tiles;
   const int total_tiles = tiles_mn * p.split_k;
-  const int t_first = blockIdx.x / CG, t_step = gridDim.x / CG;
+  const int t_first = blockIdx.x, t_step = gridDim.x;
 
   if (warp == 0) {
     // ------------------------------ TMA producer ---------------------------
@@ -310,9 +285,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     const long long pr_t0 = prof ? clock64() : 0;
     for (int t = t_first; t < total_tiles; t += t_step) {
       const int ks = t / tiles_mn, mn = t - ks * tiles_mn;
-      const int m0 = ((mn / p.n_tiles) * CG + crank) * kTileM, n0 = (mn % p.n_tiles) * BN;
+      const int m0 = (mn / p.n_tiles) * kTileM, n0 = (mn % p.n_tiles) * BN;
       const int kb0 = ks * p.kb_per_split, kb1 = min(p.kb_total, kb0 + p.kb_per_split);
-      for (int kb = kb0; kb < kb1 && !(p.debug & 2); ++kb) {
+      for (int kb = kb0; kb < kb1; ++kb) {
         const long long tw0 = prof ? clock64() : 0;
         mbar_wait(&empty_bar[s], ph ^ 1);
         if (prof) pr_wait += clock64() - tw0;
@@ -320,59 +295,19 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         uint8_t* sb = sa + kABytes;
         const int k0 = kb * TBK;
         if (elect_one()) {
-          if (CG == 2) {
-            // both CTAs load into their own shared memory; all bytes are credited to the LEADER's barrier,
-            // which the leader arms for the pair's total
-            if (crank == 0) mbar_expect_tx(&full_bar[s], 2 * (kABytes + kBBytes));
-            const uint32_t lbar = mapa_u32(&full_bar[s], 0);
-            if (A_MN) {
+          mbar_expect_tx(&full_bar[s], kABytes + kBBytes);
+          if (A_MN) {
 #pragma unroll
-              for (int c = 0; c < TBM / 64; ++c) tma_load_2d_2sm(sa + c * 8192, &map_a, lbar, m0 + c * 64, k0);
-            } else {
-              tma_load_2d_2sm(sa, &map_a, lbar, k0, m0);
-            }
-            const int nh = n0 + crank * (BN / 2);  // this CTA's half of the B tile
-            if (B_MN) {
-#pragma unroll
-              for (int c = 0; c < BN / 128; ++c) tma_load_2d_2sm(sb + c * 8192, &map_b, lbar, nh + c * 64, k0);
-            } else {
-              tma_load_2d_2sm(sb, &map_b, lbar, k0, nh);
-            }
-          } else if (p.debug & 48) {
-            // timing experiments only (results are wrong): bit 16 = B arrives on even k-blocks only, bit 32 = B never
-            // arrives: the operand bytes through the SM's memory port drop to 2/3 and 1/3 at unchanged MMA work
-            const bool with_b = (p.debug & 16) && !(kb & 1);
-            mbar_expect_tx(&full_bar[s], kABytes + (with_b ? kBBytes : 0));
-            if (A_MN) {
-#pragma unroll
-              for (int c = 0; c < kTileM / 64; ++c) tma_load_2d(sa + c * 8192, &map_a, &full_bar[s], m0 + c * 64, k0);
-            } else {
-#pragma unroll
-              for (int mi = 0; mi < TM; ++mi) tma_load_2d(sa + mi * 16384, &map_a, &full_bar[s], k0, m0 + mi * TBM);
-            }
-            if (with_b) {
-              if (B_MN) {
-#pragma unroll
-                for (int c = 0; c < BN / 64; ++c) tma_load_2d(sb + c * 8192, &map_b, &full_bar[s], n0 + c * 64, k0);
-              } else {
-                tma_load_2d(sb, &map_b, &full_bar[s], k0, n0);
-              }
-            }
+            for (int c = 0; c < kTileM / 64; ++c) tma_load_2d(sa + c * 8192, &map_a, &full_bar[s], m0 + c * 64, k0);
           } else {
-            mbar_expect_tx(&full_bar[s], kABytes + kBBytes);
-            if (A_MN) {
 #pragma unroll
-              for (int c = 0; c < kTileM / 64; ++c) tma_load_2d(sa + c * 8192, &map_a, &full_bar[s], m0 + c * 64, k0);
-            } else {
+            for (int mi = 0; mi < TM; ++mi) tma_load_2d(sa + mi * 16384, &map_a, &full_bar[s], k0, m0 + mi * TBM);
+          }
+          if (B_MN) {
 #pragma unroll
-              for (int mi = 0; mi < TM; ++mi) tma_load_2d(sa + mi * 16384, &map_a, &full_bar[s], k0, m0 + mi * TBM);
-            }
-            if (B_MN) {
-#pragma unroll
-              for (int c = 0; c < BN / 64; ++c) tma_load_2d(sb + c * 8192, &map_b, &full_bar[s], n0 + c * 64, k0);
-            } else {
-              tma_load_2d(sb, &map_b, &full_bar[s], k0, n0);
-            }
+            for (int c = 0; c < BN / 64; ++c) tma_load_2d(sb + c * 8192, &map_b, &full_bar[s], n0 + c * 64, k0);
+          } else {
+            tma_load_2d(sb, &map_b, &full_bar[s], k0, n0);
           }
         }
         __syncwarp();
@@ -382,73 +317,64 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     if (prof && lane == 0) { p.probe[24] = (unsigned long long)(clock64() - pr_t0); p.probe[25] = (unsigned long long)pr_wait; }
   } else if (warp == 1) {
     // ------------------------------ MMA issuer -----------------------------
-    if (crank == 0) {  // with CG = 2 only the pair's leader issues MMAs; whole warp loops, one elected lane issues
-      int s = 0;
-      uint32_t ph = 0;
-      int acc = 0;
-      uint32_t acc_ph = 0;
-      long long mm_wacc = 0, mm_wfull = 0;
-      const long long mm_t0 = prof ? clock64() : 0;
-      for (int t = t_first; t < total_tiles; t += t_step) {
-        const int ks = t / tiles_mn;
-        const int kb0 = ks * p.kb_per_split, kb1 = min(p.kb_total, kb0 + p.kb_per_split);
-        const bool cs_tile = CS && ((t - ks * tiles_mn) % p.n_tiles) == 0;  // column sums: once per row tile
-        const long long ta0 = prof ? clock64() : 0;
-        mbar_wait(&tmem_empty[acc], acc_ph ^ 1);
-        if (prof) mm_wacc += clock64() - ta0;
+    // the whole warp walks the loop; one elected lane issues
+    int s = 0;
+    uint32_t ph = 0;
+    int acc = 0;
+    uint32_t acc_ph = 0;
+    long long mm_wacc = 0, mm_wfull = 0;
+    const long long mm_t0 = prof ? clock64() : 0;
+    for (int t = t_first; t < total_tiles; t += t_step) {
+      const int ks = t / tiles_mn;
+      const int kb0 = ks * p.kb_per_split, kb1 = min(p.kb_total, kb0 + p.kb_per_split);
+      const bool cs_tile = CS && ((t - ks * tiles_mn) % p.n_tiles) == 0;  // column sums: once per row tile
+      const long long ta0 = prof ? clock64() : 0;
+      mbar_wait(&tmem_empty[acc], acc_ph ^ 1);
+      if (prof) mm_wacc += clock64() - ta0;
+      tc_fence_after();
+      const uint32_t d_tmem = tmem_base + (uint32_t)(acc * kAccCols);
+      for (int kb = kb0; kb < kb1; ++kb) {
+        const long long tf0 = prof ? clock64() : 0;
+        mbar_wait(&full_bar[s], ph);
+        if (prof) mm_wfull += clock64() - tf0;
         tc_fence_after();
-        const uint32_t d_tmem = tmem_base + (uint32_t)(acc * kAccCols);
-        for (int kb = kb0; kb < kb1 && !(p.debug & 2); ++kb) {
-          const long long tf0 = prof ? clock64() : 0;
-          mbar_wait(&full_bar[s], ph);
-          if (prof) mm_wfull += clock64() - tf0;
-          tc_fence_after();
-          const uint32_t sa = smem_u32(stage_base + (size_t)s * Cfg::kStageBytes);
-          const uint32_t sb = sa + kABytes;
-          // K-major: 32 bytes per UMMA_K inside the 128B swizzle row, 8-row groups 1024 B apart.
-          // MN-major: 16 k-rows (2 KB) per UMMA_K, 64-element MN chunks 8 KB apart.
-          // (the start-address field counts 16-byte units: + 2 / + 128 per UMMA_K step)
-          const uint64_t da0 = A_MN ? make_smem_desc_sw128(sa, 8192, 1024) : make_smem_desc_sw128(sa, 16, 1024);
-          const uint64_t db0 = B_MN ? make_smem_desc_sw128(sb, 8192, 1024) : make_smem_desc_sw128(sb, 16, 1024);
-          if (elect_one()) {
-#pragma unroll
-            for (int k = 0; k < TBK / UMMA_K; ++k) {
-              const uint64_t da = da0 + (uint64_t)(k * (A_MN ? 128 : 2));
-              const uint64_t db = db0 + (uint64_t)(k * (B_MN ? 128 : 2));
-              if (CG == 2) {
-                tc_mma_bf16_2sm(d_tmem, da, db, kIdesc, (kb > kb0 || k > 0) ? 1u : 0u);
-              } else {
-#pragma unroll
-                for (int mi = 0; mi < TM; ++mi)  // sub-tile mi: 16 KB (1024 descriptor units) further into the A stage
-                  tc_mma_bf16(d_tmem + (uint32_t)(mi * BN), da + (uint64_t)(mi * 1024), db, kIdesc, (kb > kb0 || k > 0) ? 1u : 0u);
-              }
-              if (CS && cs_tile) {
-                // ones tile: K-major, N = 16 rows as two aliased 8-row groups (SBO = 0), 32 bytes per UMMA_K
-                const uint64_t d1 = make_smem_desc_sw128(smem_u32(bias_s), 16, 0) + (uint64_t)(k * 2);
-#pragma unroll
-                for (int mi = 0; mi < TM; ++mi)
-                  tc_mma_bf16(tmem_base + (uint32_t)(kNAcc * kAccCols + (acc * TM + mi) * 16), da + (uint64_t)(mi * 1024), d1,
-                              make_idesc_bf16(TBM, 16, A_MN, 0), (kb > kb0 || k > 0) ? 1u : 0u);
-              }
-            }
-            if (CG == 1) tc_commit(&empty_bar[s]);  // smem stage is free once these MMAs retire
-            else tc_commit_2sm(&empty_bar[s]);      // ... in both CTAs of the pair
-          }
-          __syncwarp();
-          if (++s == kStages) { s = 0; ph ^= 1; }
-        }
+        const uint32_t sa = smem_u32(stage_base + (size_t)s * Cfg::kStageBytes);
+        const uint32_t sb = sa + kABytes;
+        // K-major: 32 bytes per UMMA_K inside the 128B swizzle row, 8-row groups 1024 B apart.
+        // MN-major: 16 k-rows (2 KB) per UMMA_K, 64-element MN chunks 8 KB apart.
+        // (the start-address field counts 16-byte units: + 2 / + 128 per UMMA_K step)
+        const uint64_t da0 = A_MN ? make_smem_desc_sw128(sa, 8192, 1024) : make_smem_desc_sw128(sa, 16, 1024);
+        const uint64_t db0 = B_MN ? make_smem_desc_sw128(sb, 8192, 1024) : make_smem_desc_sw128(sb, 16, 1024);
         if (elect_one()) {
-          if (CG == 1) tc_commit(&tmem_full[acc]);  // accumulator complete -> epilogue
-          else tc_commit_2sm(&tmem_full[acc]);
+#pragma unroll
+          for (int k = 0; k < TBK / UMMA_K; ++k) {
+            const uint64_t da = da0 + (uint64_t)(k * (A_MN ? 128 : 2));
+            const uint64_t db = db0 + (uint64_t)(k * (B_MN ? 128 : 2));
+#pragma unroll
+            for (int mi = 0; mi < TM; ++mi)  // sub-tile mi: 16 KB (1024 descriptor units) further into the A stage
+              tc_mma_bf16(d_tmem + (uint32_t)(mi * BN), da + (uint64_t)(mi * 1024), db, kIdesc, (kb > kb0 || k > 0) ? 1u : 0u);
+            if (CS && cs_tile) {
+              // ones tile: K-major, N = 16 rows as two aliased 8-row groups (SBO = 0), 32 bytes per UMMA_K
+              const uint64_t d1 = make_smem_desc_sw128(smem_u32(bias_s), 16, 0) + (uint64_t)(k * 2);
+#pragma unroll
+              for (int mi = 0; mi < TM; ++mi)
+                tc_mma_bf16(tmem_base + (uint32_t)(kNAcc * kAccCols + (acc * TM + mi) * 16), da + (uint64_t)(mi * 1024), d1,
+                            make_idesc_bf16(TBM, 16, A_MN, 0), (kb > kb0 || k > 0) ? 1u : 0u);
+            }
+          }
+          tc_commit(&empty_bar[s]);  // smem stage is free once these MMAs retire
         }
         __syncwarp();
-        if (++acc == kNAcc) { acc = 0; acc_ph ^= 1; }
+        if (++s == kStages) { s = 0; ph ^= 1; }
       }
-      if (prof && lane == 0) {
-        p.probe[8] = (unsigned long long)(clock64() - mm_t0);
-        p.probe[9] = (unsigned long long)mm_wacc;
-        p.probe[10] = (unsigned long long)mm_wfull;
-      }
+      if (elect_one()) tc_commit(&tmem_full[acc]);  // accumulator complete -> epilogue
+      __syncwarp();
+      if (++acc == kNAcc) { acc = 0; acc_ph ^= 1; }
+    }
+    if (prof && lane == 0) {
+      p.probe[8] = (unsigned long long)(clock64() - mm_t0);
+      p.probe[9] = (unsigned long long)mm_wacc;
+      p.probe[10] = (unsigned long long)mm_wfull;
     }
   } else {
     // ------------------------------ epilogue -------------------------------
@@ -460,9 +386,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     // being rewritten while an earlier store still reads it.
     // Residual (kRes): row-strided loads of the fp32 residual cost 32 L1 wavefronts per instruction (measured
     // +18 us on a 9 us GEMM), so the TMA fetches the residual block INTO the staging buffer the output will
-    // leave from -- for the NEXT tile, while this one is computed -- and the add happens in place.
+    // leave from -- for the NEXT tile, as soon as this tile's stores have been read out -- and the add happens in place.
     const int ew = warp - 2;
-    const int quad = pwarp & 3;  // TMEM lanes [32*quad, 32*quad+32): fixed by the PHYSICAL warp id
+    const int quad = warp & 3;   // TMEM lanes [32*quad, 32*quad+32)
     const int half = ew >> 2;    // columns [half*BN/2, (half+1)*BN/2)
     constexpr bool kFast = EPI >= 0;
     // Column split between the two warps of a quadrant.  128- and 256-column tiles: half each.  192-column tiles
@@ -474,7 +400,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     constexpr int NBLK = (BN / 2) / CPB;            // residual bookkeeping (fp32 output: BN / 2 columns per warp)
     constexpr int kBufs = Cfg::kStagingBufs;
     uint8_t* my_stage = staging + ew * (kBufs * 4096);
-    uint64_t* my_res_bar = res_bar + ew * 2;
+    uint64_t* my_res_bar = res_bar + ew;
     int nbuf = 0;
     int acc = 0;
     uint32_t acc_ph = 0;
@@ -489,25 +415,24 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
     const int nblk = ncols / cpb;
     const int row7 = lane & 7;
 
-    constexpr bool kResAhead = RESBUFS == 4;  // a second buffer pair: fetch a whole tile ahead
-    auto res_prefetch = [&](int t, int par) {  // lane 0: residual blocks of tile t -> buffers [NBLK par, NBLK par + NBLK)
+    auto res_prefetch = [&](int t) {  // lane 0: residual blocks of tile t -> staging buffers [0, NBLK)
       const int ks = t / tiles_mn, mn = t - ks * tiles_mn;
-      const int m0 = ((mn / p.n_tiles) * CG + crank) * kTileM, n0 = (mn % p.n_tiles) * BN;
+      const int m0 = (mn / p.n_tiles) * kTileM, n0 = (mn % p.n_tiles) * BN;
       const int nb = n0 + col_beg;
       int cnt = 0;
       for (int b = 0; b < NBLK; ++b) cnt += (nb + b * CPB < p.N) ? 1 : 0;
-      if (cnt == 0 || m0 + quad * 32 >= p.M) { mbar_arrive(&my_res_bar[par]); return; }
-      mbar_expect_tx(&my_res_bar[par], cnt * 4096);
+      if (cnt == 0 || m0 + quad * 32 >= p.M) { mbar_arrive(my_res_bar); return; }
+      mbar_expect_tx(my_res_bar, cnt * 4096);
       for (int b = 0; b < NBLK; ++b)
-        if (nb + b * CPB < p.N) tma_load_2d(my_stage + (par * NBLK + b) * 4096, &map_r, &my_res_bar[par], nb + b * CPB, m0 + quad * 32);
+        if (nb + b * CPB < p.N) tma_load_2d(my_stage + b * 4096, &map_r, my_res_bar, nb + b * CPB, m0 + quad * 32);
     };
-    if (kRes && lane == 0 && t_first < total_tiles && !(p.debug & 1)) res_prefetch(t_first, 0);
+    if (kRes && lane == 0 && t_first < total_tiles) res_prefetch(t_first);
 
     long long ep_wfull = 0, ep_wread = 0, ep_wres = 0;
     const long long ep_t0 = prof ? clock64() : 0;
     for (int t = t_first; t < total_tiles; t += t_step, ++it) {
       const int ks = t / tiles_mn, mn = t - ks * tiles_mn;
-      const int m0 = ((mn / p.n_tiles) * CG + crank) * kTileM, n0 = (mn % p.n_tiles) * BN;
+      const int m0 = (mn / p.n_tiles) * kTileM, n0 = (mn % p.n_tiles) * BN;
       ep.first_split = (ks == 0);
       const int nbeg = n0 + col_beg;
       // stage this tile's bias slice (each warp an eighth) while the accumulator is still being produced
@@ -525,20 +450,19 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
           const int mm = m0 + mi * TBM + quad * 32 + lane;
 #pragma unroll
           for (int w = 0; w < kCols / 32; ++w)
-            mk_in_all[mi][w] = (!(p.debug & 1) && mm < p.M && 32 * w < ncols && nbeg + 32 * w < p.N)
+            mk_in_all[mi][w] = (mm < p.M && 32 * w < ncols && nbeg + 32 * w < p.N)
                                    ? __ldg(p.mask_in + (size_t)((nbeg >> 5) + w) * p.M + mm) : 0u;
         }
       }
-      const int par = kResAhead ? (it & 1) : 0;
       const long long tr0 = prof ? clock64() : 0;
-      if (kRes && !(p.debug & 1)) mbar_wait(&my_res_bar[par], (uint32_t)(kResAhead ? (it >> 1) : it) & 1u);
+      if (kRes) mbar_wait(my_res_bar, (uint32_t)it & 1u);
       const long long tr1 = prof ? clock64() : 0;
       mbar_wait(&tmem_full[acc], acc_ph);
       if (prof) { ep_wres += tr1 - tr0; ep_wfull += clock64() - tr1; }
       tc_fence_after();
 #pragma unroll
       for (int mi = 0; mi < TM; ++mi) {  // the 128-row sub-tiles of the CTA tile
-      const int mrow0 = (p.debug & 1) ? p.M : m0 + mi * TBM + quad * 32;  // debug bit 0: skip all epilogue work
+      const int mrow0 = m0 + mi * TBM + quad * 32;
       const int m = mrow0 + lane;
       const bool active = mrow0 < p.M && nbeg < p.N;
       const uint32_t (&mk_in)[kCols / 32] = mk_in_all[mi];
@@ -547,31 +471,20 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       for (int b = 0; b < nblk; ++b) {
         const int n = nbeg + b * cpb;
         const bool in_range = active && n < p.N;
-        uint8_t* tile = kRes ? my_stage + (par * NBLK + b) * 4096 : my_stage + nbuf * 4096;
-        if (!in_range) {
-          if (kRes && lane == 0 && mode != kStoreDirect) bulk_commit();  // keep one bulk group per block (see wait below)
-          continue;
-        }
+        uint8_t* tile = my_stage + (kRes ? b : nbuf) * 4096;
+        if (!in_range) continue;
         uint32_t r0[32], r1[32];
         tmem_ld32(row_addr + b * cpb, r0);
         if (cpb == 64) tmem_ld32(row_addr + b * cpb + 32, r1);
-        // coalesced mode (full blocks of plain stores): the block is read back from the staging tile by the warp
-        // itself and leaves through the LSU, 4 rows x 128 B per instruction -- no bulk group to wait for, and the
-        // stores do not queue behind the operand loads in the TMA unit
-        const bool coal = !kRes && p.coalesced && mode == kStoreTma && n + cpb <= p.N;
-        if (!kRes && mode != kStoreDirect && !coal) {
+        if (!kRes && mode != kStoreDirect) {
           const long long tb0 = prof ? clock64() : 0;
-          if (lane == 0) {
-            if (p.coalesced) bulk_wait_read<0>();
-            else bulk_wait_read<kBufs - 1>();  // the store that last used this buffer has drained it
-          }
+          if (lane == 0) bulk_wait_read<kBufs - 1>();  // the store that last used this buffer has drained it
           __syncwarp();
           if (prof) ep_wread += clock64() - tb0;
         }
         tmem_ld_wait();
         const bool fast = kFast && p.vec_ok && mode != kStoreDirect && n + cpb <= p.N;
-        if (p.debug & 8) {
-        } else if (fast) {
+        if (fast) {
           uint32_t mo = 0;
           epi_math32<kFast ? EPI : 0>(ep, m, n, r0, bias_t + col_beg + b * cpb, tile + lane * 128, row7,
                                       (kFast && (EPI & kEpiMaskIn)) ? mk_in[(b * cpb) >> 5] : 0u, mo);
@@ -608,32 +521,13 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
         } else {
           stage_row_f32(tile, lane, r0);
         }
-        if (coal) {
-          __syncwarp();
-          const int esz = out_bf16 ? 2 : 4;
-          char* dbase = reinterpret_cast<char*>(ep.D) + ((int64_t)mrow0 * ep.ldd + n) * esz;
-          if (!(p.debug & 4)) {
-#pragma unroll
-            for (int i = 0; i < 8; ++i) {
-              const int row = i * 4 + (lane >> 3), chunk = lane & 7;
-              const uint4 v = *reinterpret_cast<const uint4*>(tile + row * 128 + ((chunk ^ (row & 7)) << 4));
-              if (mrow0 + row < p.M) *reinterpret_cast<uint4*>(dbase + (int64_t)row * ep.ldd * esz + chunk * 16) = v;
-            }
-          }
-          __syncwarp();  // the tile may be rewritten
-          nbuf = (nbuf + 1 == kBufs) ? 0 : nbuf + 1;
-          continue;
-        }
         fence_proxy_async();
         __syncwarp();
         if (lane == 0) {
-          if (p.debug & 4) {
-          } else if (mode == kStoreTmaAdd) tma_reduce_add_2d(&map_d, tile, n, mrow0);
+          if (mode == kStoreTmaAdd) tma_reduce_add_2d(&map_d, tile, n, mrow0);
           else tma_store_2d(&map_d, tile, n, mrow0);
           bulk_commit();
-          if (!kRes && p.coalesced) bulk_wait_read<0>();  // (ragged block in coalesced mode: free the tile at once)
         }
-        if (!kRes && p.coalesced) __syncwarp();
         if (!kRes) nbuf = (nbuf + 1 == kBufs) ? 0 : nbuf + 1;
       }
       if (CS && n0 == 0 && half == 0 && mrow0 < p.M) {
@@ -646,21 +540,11 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       tc_fence_before();
       __syncwarp();
       if (lane == 0) {
-        if (CG == 1) mbar_arrive(&tmem_empty[acc]);
-        else mbar_arrive_cluster(mapa_u32(&tmem_empty[acc], 0));  // the leader's MMA thread waits for both CTAs
-        if (kRes && !(p.debug & 1)) {
-          // residual of the next tile -> the other buffer pair, once the stores of the PREVIOUS tile (which
-          // left from that pair) have been read out; this tile's NBLK groups may still be in flight
-          const int tn = t + t_step;
-          if (tn < total_tiles) {
-            if (kResAhead) {
-              bulk_wait_read<NBLK>();
-              res_prefetch(tn, par ^ 1);
-            } else {
-              bulk_wait_read<0>();  // same buffers: this tile's stores must have been read out
-              res_prefetch(tn, 0);
-            }
-          }
+        mbar_arrive(&tmem_empty[acc]);
+        if (kRes && t + t_step < total_tiles) {
+          // residual of the next tile -> the same buffers, once this tile's stores have been read out of them
+          bulk_wait_read<0>();
+          res_prefetch(t + t_step);
         }
       }
       if (++acc == kNAcc) { acc = 0; acc_ph ^= 1; }
@@ -678,11 +562,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 
   tc_fence_before();
   __syncthreads();
-  if (CG == 2) cluster_sync_all();  // neither CTA may free TMEM / retire while the pair's MMAs or arrives are in flight
   if (warp == 1) {
     tc_fence_after();
-    if (CG == 1) tmem_dealloc<Cfg::kTmemCols>(tmem_base);
-    else tmem_dealloc_2sm<Cfg::kTmemCols>(tmem_base);
+    tmem_dealloc<Cfg::kTmemCols>(tmem_base);
   }
   clock_probe_end(p.probe);
 }
@@ -741,11 +623,15 @@ int make_tmap_bf16_2d(CUtensorMap* map, const void* base, int64_t inner, int64_t
   return make_tmap_2d(map, base, DGPT_BF16, inner, outer, ld, 64, box_outer);
 }
 
-template <int BN, int A_MN, int B_MN, int EPI, int OBF, int CG, int RESBUFS, int CS = 0, int TM = 1>
-static int launch_one(const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& md, const CUtensorMap& mr,
-                      const TcParams& p, int grid, cudaStream_t st) {
-  using Cfg = TcCfg<BN, CG, RESBUFS, CS, TM>;
-  auto kern = gemm_tc_kernel<BN, A_MN, B_MN, EPI, OBF, CG, RESBUFS, CS, TM>;
+struct TcMaps {
+  CUtensorMap a, b, d, r;
+};
+
+// persistent grid: one CTA per SM, or one per tile when there are fewer tiles
+template <int BN, int A_MN, int B_MN, int EPI, int OBF, int CS = 0, int TM = 1>
+static int launch_one(const TcMaps& m, const TcParams& p, int sms, cudaStream_t st) {
+  using Cfg = TcCfg<BN, EPI, CS, TM>;
+  auto kern = gemm_tc_kernel<BN, A_MN, B_MN, EPI, OBF, CS, TM>;
   static bool attr_done = false;
   if (!attr_done) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)Cfg::kSmemBytes);
@@ -756,53 +642,21 @@ static int launch_one(const CUtensorMap& ma, const CUtensorMap& mb, const CUtens
     attr_done = true;
   }
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
+  cfg.gridDim = dim3((unsigned)min(p.m_tiles * p.n_tiles * p.split_k, sms));
   cfg.blockDim = dim3(kThreads);
   cfg.dynamicSmemBytes = Cfg::kSmemBytes;
   cfg.stream = st;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CG;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[1].val.programmaticStreamSerializationAllowed = 1;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = pdl_enabled() ? 2 : 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, ma, mb, md, mr, p);
+  cfg.numAttrs = pdl_enabled() ? 1 : 0;
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, m.a, m.b, m.d, m.r, p);
   if (e != cudaSuccess) {
     set_error("gemm_tc: launch: %s", cudaGetErrorString(e));
     return DGPT_E_LAUNCH;
   }
   return check_launch("gemm_tc");
-}
-
-// Pair tiles (cta_group::2) are opt-in (dgpt_gemm_set_cta_group / DGPT_GEMM_CTA_GROUP=2): on the model's shapes
-// the single-CTA mainloop already runs at the SM's 64 B/cycle operand-ingest limit and pairs measured at most
-// 5 % faster in the mainloop and slower end to end, so the default stays 1.
-static int g_cta_group = -1;  // -1: not set yet (DGPT_GEMM_CTA_GROUP, default 1)
-void set_gemm_cta_group(int g) { g_cta_group = (g == 2) ? 2 : 1; }
-static int gemm_cta_group() {
-  if (g_cta_group < 0) {
-    const char* e = getenv("DGPT_GEMM_CTA_GROUP");
-    g_cta_group = (e && atoi(e) == 2) ? 2 : 1;
-  }
-  return g_cta_group;
-}
-
-struct TcMaps {
-  CUtensorMap a, b, b_half, d, r;
-};
-
-// pair tiles whenever requested and the row-tile count is even, single-CTA tiles otherwise
-template <int BN, int A_MN, int B_MN, int EPI, int OBF, int RESBUFS = 0>
-static int launch_cfg(const TcMaps& m, const TcParams& p, int sms, cudaStream_t st) {
-  if (p.cta_group == 2 && BN != 192) {
-    const int total = (p.m_tiles / 2) * p.n_tiles * p.split_k;
-    return launch_one<BN, A_MN, B_MN, EPI, OBF, 2, RESBUFS>(m.a, m.b_half, m.d, m.r, p, 2 * min(total, sms / 2), st);
-  }
-  const int total = p.m_tiles * p.n_tiles * p.split_k;
-  return launch_one<BN, A_MN, B_MN, EPI, OBF, 1, RESBUFS>(m.a, m.b, m.d, m.r, p, min(total, sms), st);
 }
 
 int launch_gemm_tc(const dgpt_gemm_args* a, cudaStream_t st) {
@@ -812,11 +666,6 @@ int launch_gemm_tc(const dgpt_gemm_args* a, cudaStream_t st) {
   // tile N: widest tile that still yields >= ~1 wave of CTAs
   int sms = dgpt_sm_count();
   if (sms <= 0) sms = 148;
-  {  // DGPT_GEMM_SMS: leave some SMs to concurrently running kernels (the NCCL all-reduce of the data-parallel step)
-    static int cap = -1;
-    if (cap < 0) { const char* e = getenv("DGPT_GEMM_SMS"); cap = e ? atoi(e) : 0; }
-    if (cap > 0 && cap < sms) sms = cap;
-  }
   int m_tiles = ceil_div(a->M, TBM);
   // 128 x 256 tiles ingest 25 % fewer operand bytes per MMA cycle than 128 x 128; a ragged last column
   // tile (N = 1152 -> 4.5 tiles) costs less than that as soon as N >= 1024 (TMA zero-fills, the store clips)
@@ -824,19 +673,15 @@ int launch_gemm_tc(const dgpt_gemm_args* a, cudaStream_t st) {
   // wgrads that carry a column sum (bias gradient): 256-column tiles when the output has few row tiles and wide rows
   // (FFN2: 384 x 1536) -- a 128 x 128 tile needs 64 operand bytes per 1 K MMA cycles where the SM ingests ~70 B/cycle,
   // a 128 x 256 tile 48; their single accumulator buffer costs nothing because a split-K CTA owns one tile.
-  // DGPT_GEMM_CS256=0 keeps 128-column tiles (Runner._splits reads the same variable).
-  static int cs256_env = -1;
-  if (cs256_env < 0) { const char* e = getenv("DGPT_GEMM_CS256"); cs256_env = e ? atoi(e) : 1; }
-  const bool cs_wide = cs256_env && a->a_colsum && a->N % 256 == 0 && a->N >= 512 && m_tiles < 8;
+  // (Runner._splits mirrors this rule when it picks the wgrad split count.)
+  const bool cs_wide = a->a_colsum && a->N % 256 == 0 && a->N >= 512 && m_tiles < 8;
   if (a->N <= 128 || (a->N % 256 != 0 && a->N < 1024) || (a->a_colsum && !cs_wide)) BN = 128;
   if (BN == 256 && !cs_wide && m_tiles * ceil_div(a->N, 256) * (a->split_k > 1 ? a->split_k : 1) < sms) BN = 128;
   // 192-column tiles for N = 192, 384, 576, 960 (the model's N = 384 GEMMs): two tiles per row instead of three
-  static int bn192_env = -1;
-  if (bn192_env < 0) { const char* e = getenv("DGPT_GEMM_BN192"); bn192_env = e ? atoi(e) : 1; }
   // (measured: ~5 % faster for the dgrad / wgrad GEMMs with >= 8 row tiles; slower with the residual epilogue, whose
   // three staging buffers per warp leave a 3-stage ring, and for small wgrads that would need > 20 K splits)
   // (the bit-mask epilogues are instantiated for 128- / 256-column tiles only)
-  if (bn192_env && BN == 128 && a->N % 192 == 0 && a->N % 256 != 0 && a->N < 1024 && m_tiles >= 8 && !a->residual &&
+  if (BN == 128 && a->N % 192 == 0 && a->N % 256 != 0 && a->N < 1024 && m_tiles >= 8 && !a->residual &&
       !a->relu_mask_in && !a->relu_mask_out)
     BN = 192;
   // Wave quantisation for the big-activation GEMMs (M >= 1024 rows, no split-K): a persistent grid of `sms` CTAs walks
@@ -844,10 +689,8 @@ int launch_gemm_tc(const dgpt_gemm_args* a, cudaStream_t st) {
   // 81 % empty, and N = 1152 wastes half of every fifth column tile on top.  Pick the width with the best
   //   (useful columns / tiled columns) * (tiles / (rounds * sms)) * (tile-shape factor: 1.0 / 0.95 / 0.88 for 256 / 192 / 128,
   // measured: operand re-reads and per-tile bookkeeping).  FFN1 fwd / FFN2 dgrad (N = 1536): 192 (1024 tiles, 6.9 rounds);
-  // QKV fwd (N = 1152): 128 (1152 tiles, 7.8 rounds).  DGPT_GEMM_WAVE=0 turns the rule off.
-  static int wave_env = -1;
-  if (wave_env < 0) { const char* e = getenv("DGPT_GEMM_WAVE"); wave_env = e ? atoi(e) : 1; }
-  if (wave_env && BN == 256 && !cs_wide && a->split_k <= 1 && m_tiles >= 8 && !a->residual && !a->a_colsum && a->N >= 1024) {
+  // QKV fwd (N = 1152): 128 (1152 tiles, 7.8 rounds).
+  if (BN == 256 && !cs_wide && a->split_k <= 1 && m_tiles >= 8 && !a->residual && !a->a_colsum && a->N >= 1024) {
     auto score = [&](int bn, double shape) {
       const int nt = ceil_div(a->N, bn), tiles = m_tiles * nt, rounds = ceil_div(tiles, sms);
       return shape * ((double)a->N / (nt * bn)) * ((double)tiles / ((double)rounds * sms));
@@ -856,22 +699,15 @@ int launch_gemm_tc(const dgpt_gemm_args* a, cudaStream_t st) {
     if (a->N % 192 == 0 && score(192, 0.95) > best) { best = score(192, 0.95); BN = 192; }
     if (score(128, 0.88) > best) BN = 128;
   }
-  {  // DGPT_GEMM_FORCE_BN=128|256: tile-width experiments (192 only through the rule above)
-    static int force = -1;
-    if (force < 0) { const char* e = getenv("DGPT_GEMM_FORCE_BN"); force = e ? atoi(e) : 0; }
-    if ((force == 128 || force == 256) && !a->a_colsum && !(force == 256 && a->residual)) BN = force;
-  }
   // 256-row CTA tiles (TM = 2: two M = 128 MMAs per k-step on one B stage, 1/3 fewer operand bytes per MMA cycle) for
   // the forward / dgrad GEMMs of the model's big activations: plain, bias + ReLU (+ mask) and mask-in epilogues with
-  // bf16 output, no split-K, no residual (the TMA-fed residual path is a 128-row design).  DGPT_GEMM_TM=1 turns it off.
-  static int tm_env = -1;
-  if (tm_env < 0) { const char* e = getenv("DGPT_GEMM_TM"); tm_env = e ? atoi(e) : 0; }
-  int TM = 1;
-  // measured (profiles/r2_gemm_experiments.txt): 256-row tiles are 3 % faster for K >= 1024 (FFN1 / QKV dgrad) and
+  // bf16 output, no split-K, no residual (the TMA-fed residual path is a 128-row design).
+  // Measured (profiles/r2_gemm_experiments.txt): 256-row tiles are 3 % faster for K >= 1024 (FFN1 / QKV dgrad) and
   // 10-20 % SLOWER for the K = 384 GEMMs, whose pace is set by the epilogue (single-buffered accumulators serialise it
-  // with the mainloop): default = 256-row tiles only for K >= 1024; DGPT_GEMM_TM=1 never, =2 whenever instantiated
-  if ((tm_env == 2 || (tm_env == 0 && a->K >= 1024)) && !a_mn && a->M >= 1024 && a->d_dtype == DGPT_BF16 && !a->residual && !a->D2 && !a->relu_aux &&
-      a->dropout_p == 0.f && a->split_k <= 1 && !a->accumulate && !a->a_colsum && gemm_cta_group() == 1) {
+  // with the mainloop): 256-row tiles only for K >= 1024.
+  int TM = 1;
+  if (a->K >= 1024 && !a_mn && a->M >= 1024 && a->d_dtype == DGPT_BF16 && !a->residual && !a->D2 && !a->relu_aux &&
+      a->dropout_p == 0.f && a->split_k <= 1 && !a->accumulate && !a->a_colsum) {
     // tile width for 256-row tiles: 192 when it divides N (N = 384, 1152: no ragged column tile), else 256
     const int bn2 = (a->N % 192 == 0 && a->N % 256 != 0) ? 192 : (a->N >= 256 ? 256 : 0);
     // only the fast-path epilogues the model uses are instantiated for 256-row tiles (TMA-addressable bf16 output,
@@ -902,35 +738,18 @@ int launch_gemm_tc(const dgpt_gemm_args* a, cudaStream_t st) {
   }
   auto al16 = [](const void* q) { return ((uintptr_t)q & 15) == 0; };
   p.vec_ok = (a->N % 4 == 0) && (!a->bias || al16(a->bias)) && (!a->residual || (al16(a->residual) && a->ldr % 4 == 0));
-  {
-    static int role_hi = -1;
-    if (role_hi < 0) { const char* e = getenv("DGPT_GEMM_ROLE_HI"); role_hi = e ? atoi(e) : 0; }
-    p.role_hi = role_hi;
-    static int coal = -1;
-    if (coal < 0) { const char* e = getenv("DGPT_GEMM_STORE"); coal = (e && e[0] == 'c') ? 1 : 0; }
-    p.coalesced = coal;
-  }
   p.mask_out = a->relu_mask_out;
   p.mask_in = a->relu_mask_in;
   p.a_colsum = a->a_colsum;
-  {
-    static int dbg = -1;
-    if (dbg < 0) { const char* e = getenv("DGPT_GEMM_DEBUG"); dbg = e ? atoi(e) : 0; }
-    p.debug = dbg;
-    p.probe = clock_probe_buffer();
-  }
+  p.probe = clock_probe_buffer();
   TcMaps mp;
   int rc;
   if (a_mn) rc = make_tmap_bf16_2d(&mp.a, a->A, a->M, a->K, a->lda, 64);
   else rc = make_tmap_bf16_2d(&mp.a, a->A, a->K, a->M, a->lda, TBM);
   if (rc) return rc;
-  // b_half: B as loaded by one CTA of a pair (half of the tile's rows)
   if (b_mn) rc = make_tmap_bf16_2d(&mp.b, a->B, a->N, a->K, a->ldb, 64);
   else rc = make_tmap_bf16_2d(&mp.b, a->B, a->K, a->N, a->ldb, BN);
   if (rc) return rc;
-  if (b_mn) mp.b_half = mp.b;
-  else if ((rc = make_tmap_bf16_2d(&mp.b_half, a->B, a->K, a->N, a->ldb, BN / 2))) return rc;
-  p.cta_group = (TM == 1 && gemm_cta_group() == 2 && m_tiles % 2 == 0) ? 2 : 1;
   // output through TMA when its pitch allows it (always true for the model's buffers)
   const int desz = a->d_dtype == DGPT_F32 ? 4 : 2;
   p.store_mode = kStoreDirect;
@@ -968,12 +787,8 @@ int launch_gemm_tc(const dgpt_gemm_args* a, cudaStream_t st) {
       if ((rc = make_tmap_2d(&mp.r, a->residual, DGPT_F32, a->N, a->M, a->ldr, 32, 32))) return rc;
     }
   }
-  // residual staging buffers per epilogue warp (see TcCfg)
-  static int res_bufs_env = -1;
-  if (res_bufs_env < 0) { const char* e = getenv("DGPT_GEMM_RES_BUFS"); res_bufs_env = e ? atoi(e) : 0; }
-  const int res_bufs = res_bufs_env == 4 ? 4 : 2;  // measured: 2 is never slower (DGPT_GEMM_RES_BUFS=4 for experiments)
 #define TC_EPI(BN_, A_, B_, E_, O_) \
-  if (epi == (E_) && obf == (O_)) return launch_cfg<BN_, A_, B_, (E_), O_>(mp, p, sms, st);
+  if (epi == (E_) && obf == (O_)) return launch_one<BN_, A_, B_, (E_), O_>(mp, p, sms, st);
 #define TC_DISPATCH(BN_)                                                              \
   if (BN == BN_) {                                                                    \
     if (!a_mn && !b_mn) {                                                             \
@@ -981,38 +796,28 @@ int launch_gemm_tc(const dgpt_gemm_args* a, cudaStream_t st) {
       if (BN_ == 128) { TC_EPI(128, 0, 0, kEpiBias, 0) }  /* lm_head: fp32 logits, N = 80 (full blocks fast) */ \
       TC_EPI(BN_, 0, 0, kEpiBias | kEpiRelu, 1)                                       \
       TC_EPI(BN_, 0, 0, kEpiBias | kEpiRelu | kEpiMaskOut, 1)                         \
-      if (BN_ == 128 && epi >= 0 && (epi & kEpiRes)) {                                \
-        const bool ahead = res_bufs == 4;                                             \
-        if (epi == (kEpiBias | kEpiRes))                                              \
-          return ahead ? launch_cfg<128, 0, 0, kEpiBias | kEpiRes, 0, 4>(mp, p, sms, st)              \
-                       : launch_cfg<128, 0, 0, kEpiBias | kEpiRes, 0, 2>(mp, p, sms, st);             \
-        if (epi == (kEpiBias | kEpiDrop | kEpiRes))                                   \
-          return ahead ? launch_cfg<128, 0, 0, kEpiBias | kEpiDrop | kEpiRes, 0, 4>(mp, p, sms, st)   \
-                       : launch_cfg<128, 0, 0, kEpiBias | kEpiDrop | kEpiRes, 0, 2>(mp, p, sms, st);  \
-        epi = -1;                                                                     \
+      if (BN_ == 128) {                                                               \
+        TC_EPI(128, 0, 0, kEpiBias | kEpiRes, 0)                                      \
+        TC_EPI(128, 0, 0, kEpiBias | kEpiDrop | kEpiRes, 0)                           \
       }                                                                               \
-      return launch_cfg<BN_, 0, 0, -1, 0>(mp, p, sms, st);                            \
+      return launch_one<BN_, 0, 0, -1, 0>(mp, p, sms, st);                            \
     }                                                                                 \
     if (!a_mn && b_mn) {                                                              \
       TC_EPI(BN_, 0, 1, 0, 1)                                                         \
       TC_EPI(BN_, 0, 1, 0, 0)                                                         \
       TC_EPI(BN_, 0, 1, kEpiMaskIn, 1)                                                \
-      return launch_cfg<BN_, 0, 1, -1, 0>(mp, p, sms, st);                            \
+      return launch_one<BN_, 0, 1, -1, 0>(mp, p, sms, st);                            \
     }                                                                                 \
     if (a->a_colsum) {                                                                \
       DGPT_REQUIRE(epi == 0 && obf == 0, "gemm(bf16): a_colsum needs the plain fp32 wgrad form");   \
-      const int total = p.m_tiles * p.n_tiles * p.split_k;                            \
-      return launch_one<BN_, 1, 1, 0, 0, 1, 0, 1>(mp.a, mp.b, mp.d, mp.r, p, min(total, sms), st);               \
+      return launch_one<BN_, 1, 1, 0, 0, 1>(mp, p, sms, st);                          \
     }                                                                                 \
     TC_EPI(BN_, 1, 1, 0, 0)                                                           \
-    return launch_cfg<BN_, 1, 1, -1, 0>(mp, p, sms, st);                              \
+    return launch_one<BN_, 1, 1, -1, 0>(mp, p, sms, st);                              \
   }
   if (TM == 2) {
-    const int grid = min(p.m_tiles * p.n_tiles, sms);
-    const bool masks_ok = true;
 #define TC_TM2(BN_, B_, E_) \
-    if (BN == (BN_) && b_mn == (B_) && epi == (E_) && obf == 1 && masks_ok) \
-      return launch_one<BN_, 0, B_, (E_), 1, 1, 0, 0, 2>(mp.a, mp.b, mp.d, mp.r, p, grid, st);
+    if (BN == (BN_) && b_mn == (B_) && epi == (E_) && obf == 1) return launch_one<BN_, 0, B_, (E_), 1, 0, 2>(mp, p, sms, st);
     TC_TM2(256, 0, 0)
     TC_TM2(256, 0, kEpiBias | kEpiRelu | kEpiMaskOut)
     TC_TM2(256, 0, kEpiBias | kEpiRelu)
@@ -1024,26 +829,23 @@ int launch_gemm_tc(const dgpt_gemm_args* a, cudaStream_t st) {
     set_error("gemm_tc: internal: no 256-row instantiation for BN=%d b_mn=%d epi=%d", BN, b_mn, epi);
     return DGPT_E_ARG;
   }
-  if (BN == 192) {  // single-CTA tiles only; the instantiations the N = 384 GEMMs of the model need, else generic
-    p.cta_group = 1;
-    const int grid = min(p.m_tiles * p.n_tiles * p.split_k, sms);
-#define TC_192(A_, B_, E_, O_, R_, C_) \
+  if (BN == 192) {  // the instantiations the N = 384 GEMMs of the model need, else generic
+#define TC_192(A_, B_, E_, O_, C_) \
     if (a_mn == (A_) && b_mn == (B_) && epi == (E_) && obf == (O_) && (a->a_colsum != nullptr) == ((C_) != 0)) \
-      return launch_one<192, A_, B_, (E_), O_, 1, R_, C_>(mp.a, mp.b, mp.d, mp.r, p, grid, st);
-    TC_192(0, 0, 0, 1, 0, 0)
-    TC_192(0, 0, kEpiBias | kEpiRelu, 1, 0, 0)
-    TC_192(0, 0, kEpiBias | kEpiRelu | kEpiMaskOut, 1, 0, 0)
-    TC_192(0, 1, kEpiMaskIn, 1, 0, 0)
-    TC_192(0, 1, 0, 1, 0, 0)
-    TC_192(0, 1, 0, 0, 0, 0)
-    TC_192(1, 1, 0, 0, 0, 0)
-    TC_192(1, 1, 0, 0, 0, 1)
+      return launch_one<192, A_, B_, (E_), O_, C_>(mp, p, sms, st);
+    TC_192(0, 0, 0, 1, 0)
+    TC_192(0, 0, kEpiBias | kEpiRelu, 1, 0)
+    TC_192(0, 0, kEpiBias | kEpiRelu | kEpiMaskOut, 1, 0)
+    TC_192(0, 1, kEpiMaskIn, 1, 0)
+    TC_192(0, 1, 0, 1, 0)
+    TC_192(0, 1, 0, 0, 0)
+    TC_192(1, 1, 0, 0, 0)
+    TC_192(1, 1, 0, 0, 1)
 #undef TC_192
     DGPT_REQUIRE(!a->a_colsum, "gemm(bf16): a_colsum needs the plain fp32 wgrad form");
-    if (epi >= 0 && (epi & kEpiRes)) epi = -1;
-    if (!a_mn && !b_mn) return launch_one<192, 0, 0, -1, 0, 1, 0, 0>(mp.a, mp.b, mp.d, mp.r, p, grid, st);
-    if (!a_mn && b_mn) return launch_one<192, 0, 1, -1, 0, 1, 0, 0>(mp.a, mp.b, mp.d, mp.r, p, grid, st);
-    return launch_one<192, 1, 1, -1, 0, 1, 0, 0>(mp.a, mp.b, mp.d, mp.r, p, grid, st);
+    if (!a_mn && !b_mn) return launch_one<192, 0, 0, -1, 0>(mp, p, sms, st);
+    if (!a_mn && b_mn) return launch_one<192, 0, 1, -1, 0>(mp, p, sms, st);
+    return launch_one<192, 1, 1, -1, 0>(mp, p, sms, st);
   }
   TC_DISPATCH(128)
   TC_DISPATCH(256)

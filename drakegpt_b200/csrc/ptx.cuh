@@ -99,63 +99,6 @@ __device__ __forceinline__ void tma_load_3d(void* dst, const CUtensorMap* map, u
       : "memory");
 }
 
-// ---- 2-CTA (cta_group::2) helpers: the pair shares one MMA; barriers of the leader (rank 0) are reached
-// through shared::cluster addresses -------------------------------------------------------------------
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared::cluster address of `p` (a shared-memory object of this CTA) in CTA `rank` of the cluster
-__device__ __forceinline__ uint32_t mapa_u32(const void* p, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_u32(p)), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA load into THIS CTA's shared memory whose byte count is credited to a barrier of the pair's leader
-__device__ __forceinline__ void tma_load_2d_2sm(void* dst, const CUtensorMap* map, uint32_t leader_bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(leader_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-template <int kCols>
-__device__ __forceinline__ void tmem_alloc_2sm(uint32_t* smem_dst) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(smem_dst)), "n"(kCols)
-               : "memory");
-  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-template <int kCols>
-__device__ __forceinline__ void tmem_dealloc_2sm(uint32_t taddr) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "n"(kCols) : "memory");
-}
-// arrives on the barrier at this offset in both CTAs of the pair once the pair's MMAs have retired
-__device__ __forceinline__ void tc_commit_2sm(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::"r"(
-                   smem_u32(bar)),
-               "h"((uint16_t)0x3)
-               : "memory");
-}
-// D[tmem of both CTAs] (+)= A (128 rows from each CTA) * B (N/2 rows from each CTA); issued by the leader only
-__device__ __forceinline__ void tc_mma_bf16_2sm(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc,
-                                                uint32_t accumulate) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t"
-      "}\n" ::"r"(d_tmem),
-      "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
 // contiguous global -> shared bulk copy (no tensor map); size and both addresses multiples of 16 bytes
 __device__ __forceinline__ void bulk_load_1d(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(

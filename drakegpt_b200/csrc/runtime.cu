@@ -77,7 +77,7 @@ int require_device() {
 extern "C" {
 
 const char* dgpt_last_error(void) { return dgpt::g_err; }
-int dgpt_abi_version(void) { return 1; }
+int dgpt_abi_version(void) { return 2; }
 
 int dgpt_device_check(void) { return dgpt::require_device(); }
 

@@ -403,10 +403,8 @@ class Runner:
     def _splits(n_out_rows, n_out_cols, k, sm, colsum=False):
         # column tile of the wgrad GEMM: 192 for N = 192 / 384 / 576 / 960, 256 for a wide output with few row tiles that
         # also carries a column sum (FFN2: 384 x 1536), else 128 (launch_gemm_tc picks the same)
-        import os
         bn = 192 if (n_out_cols % 192 == 0 and n_out_cols % 256 != 0 and n_out_cols < 1024 and n_out_rows >= 1024) else 128
-        if (colsum and n_out_cols % 256 == 0 and n_out_cols >= 512 and n_out_rows < 1024
-                and os.environ.get("DGPT_GEMM_CS256", "1") != "0"):
+        if colsum and n_out_cols % 256 == 0 and n_out_cols >= 512 and n_out_rows < 1024:
             bn = 256
         tiles = ((n_out_rows + 127) // 128) * ((n_out_cols + bn - 1) // bn)
         return max(1, min(sm // max(tiles, 1), k // 512))

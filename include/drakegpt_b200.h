@@ -160,9 +160,6 @@ typedef struct dgpt_gemm_args {
   float* a_colsum;
 } dgpt_gemm_args;
 int dgpt_gemm(const dgpt_gemm_args* a, void* stream);
-/* Tensor-mode tiling knob: 1 (default) = one CTA per 128-row tile; 2 = CTA pairs (thread-block cluster of 2,
- * tcgen05 cta_group::2, 256-row pair tiles, each CTA stages half of B).  Process-wide; returns DGPT_E_ARG otherwise. */
-int dgpt_gemm_set_cta_group(int cta_group);
 
 /* out[n] (+)= sum_m X[m,n]   (bias gradients) */
 int dgpt_colsum(const void* X, int dtype, int M, int N, int ldx, float* out, int accumulate,

@@ -103,30 +103,6 @@ def test_gemm_tcgen05_vs_fp32(M, N, K, amaj, bmaj):
     assert err <= 2e-3 * math.sqrt(K), (err, M, N, K, amaj, bmaj)
 
 
-def test_gemm_tcgen05_cta_pairs():
-    """cta_group::2 pair tiles (opt-in) give the same results as single-CTA tiles."""
-    g = torch.Generator().manual_seed(77)
-    L = _lib.lib()
-    try:
-        for (M, N, K, amaj, bmaj) in [(512, 384, 256, MAJOR_K, MAJOR_K), (256, 1536, 384, MAJOR_K, MAJOR_MN),
-                                      (1536, 384, 1024, MAJOR_MN, MAJOR_MN)]:
-            A, Bm = torch.randn(M, K, generator=g).bfloat16(), torch.randn(N, K, generator=g).bfloat16()
-            Ad = (A if amaj == MAJOR_K else A.t().contiguous()).to(DEV)
-            Bd = (Bm if bmaj == MAJOR_K else Bm.t().contiguous()).to(DEV)
-            outs = []
-            for cg in (1, 2):
-                assert L.dgpt_gemm_set_cta_group(cg) == 0
-                out = torch.full((M, N), float("nan"), device=DEV)
-                ops.raw_gemm(Ad, Bd, out, a_major=amaj, b_major=bmaj, M=M, N=N, K=K)
-                outs.append(out.cpu())
-            ref = A.float() @ Bm.float().t()
-            assert (outs[1] - ref).abs().max() <= 2e-3 * math.sqrt(K)
-            torch.testing.assert_close(outs[0], outs[1], rtol=1e-4, atol=1e-3)
-        assert L.dgpt_gemm_set_cta_group(3) != 0
-    finally:
-        L.dgpt_gemm_set_cta_group(1)
-
-
 def test_gemm_tcgen05_epilogue_and_splitk():
     g = torch.Generator().manual_seed(21)
     M, N, K, p, seed, site = 256, 384, 512, 0.2, 99, 5

@@ -11,6 +11,7 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from drakegpt_b200 import ops
 from drakegpt_b200._lib import MAJOR_K, MAJOR_MN
+from drakegpt_b200.engine import Runner
 
 dev = "cuda"
 shapes = {  # name: (M, N, K, a_major, b_major, out dtype, epilogue)
@@ -33,14 +34,6 @@ which = args or list(shapes)
 R = int(os.environ.get('GEMM_PROBE_R', '6'))  # operand / output sets (1: everything L2-resident)
 
 
-def splits(rows, cols, k, sm=148):
-    bn = 192 if (cols % 192 == 0 and cols % 256 != 0 and cols < 1024 and rows >= 1024) else 128
-    if os.environ.get("DGPT_GEMM_BN192") == "0":
-        bn = 128
-    tiles = ((rows + 127) // 128) * ((cols + bn - 1) // bn)
-    return max(1, min(sm // max(tiles, 1), k // 512))
-
-
 def make(name):
     M, N, K, am, bm, odt, epi = shapes[name]
     A = torch.randn((M, K) if am == MAJOR_K else (K, M), device=dev).bfloat16()
@@ -54,7 +47,7 @@ def make(name):
     elif epi == "relu_aux":
         kw = dict(relu_mask_in=torch.randint(-2**31, 2**31 - 1, ((N // 32) * M,), device=dev, dtype=torch.int32))
     elif epi == "splitk":
-        kw = dict(accumulate=True, split_k=splits(M, N, K))
+        kw = dict(accumulate=True, split_k=Runner._splits(M, N, K, ops.sm_count()))
     return lambda: ops.raw_gemm(A, B, out, a_major=am, b_major=bm, **kw)
 
 
