@@ -20,7 +20,7 @@ EXPORTS = [
     "dgpt_attn_bwd", "dgpt_attn_bwd_scratch_bytes", "dgpt_cross_entropy", "dgpt_lmhead_ce", "dgpt_lmhead_ce_supported", "dgpt_gemm_res_ln", "dgpt_gemm_res_ln_supported", "dgpt_adamw", "dgpt_counter_add", "dgpt_sample",
     "dgpt_ipc_export", "dgpt_ipc_open", "dgpt_ipc_close", "dgpt_peer_copy", "dgpt_dp_adamw",
     "dgpt_decode_attn", "dgpt_decode_persistent", "dgpt_decode_persistent_scratch_floats",
-    "dgpt_decode_persistent_max_batch",
+    "dgpt_decode_persistent_max_batch", "dgpt_sample_ex", "dgpt_decode_persistent_ex",
 ]
 
 
@@ -102,6 +102,9 @@ def _declare(lib):
         "dgpt_peer_copy": [vp, vp, i64, vp],
         "dgpt_dp_adamw": [C.POINTER(C.c_void_p), i32, i32, vp, vp, i64, i64, vp, vp, vp, vp, i32, vp],
         "dgpt_sample": [vp, i32, vp, i64, i32, i32, i32, i32, u64, vp, u32, vp],
+        "dgpt_sample_ex": [vp, i32, vp, i64, i32, i32, i32, i32, u64, vp, u32, vp, vp],
+        "dgpt_decode_persistent_ex": [C.POINTER(C.c_void_p), i32, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32,
+                                      i32, i32, i32, i32, i32, u64, vp, vp, i32, vp],
     }
     for name, args in sig.items():
         fn = getattr(lib, name)

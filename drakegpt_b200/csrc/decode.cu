@@ -10,13 +10,14 @@
 //   decode_persistent_kernel  small batches (<= 8 sequences): ONE launch generates every token of the in-window part.
 //                             All layers of a token run as phases of a persistent grid (LayerNorm fused into the
 //                             matrix-vector prologue, bias / ReLU / residual into its epilogue, KV append, attention,
-//                             LM head, on-device multinomial / argmax sampling) separated by cluster barriers;
+//                             LM head, on-device sampling: warp_sample_row of sample.cuh) separated by cluster barriers;
 //                             the 21.6 MB of bf16 weights stay L2-resident across tokens.  The launch-per-kernel path
 //                             needs ~45 launches per token; this one needs none.
 #include <cuda.h>
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "sample.cuh"
 
 namespace dgpt {
 
@@ -199,6 +200,7 @@ struct DecP {
   int greedy;
   uint64_t seed;
   const uint64_t* seed_dev;
+  const dgpt_sampling* sampling;  // NULL: plain multinomial
   float eps;
   unsigned long long* probe;    // DGPT_CLOCK_PROBE: phase stamps of the last position (cluster 0, CTA 0)
 };
@@ -450,6 +452,7 @@ __global__ void __launch_bounds__(kPThreads, 1) decode_persistent_kernel(DecP p)
   float* red = lg + BM * V;           // [32 + 8 * 64] attention reductions
   float* qs = red + 32 + 8 * kDecH;   // [64] query of the (sequence, head) in flight
   float* ao = qs + kDecH;             // [64] attention output of it
+  float* ss = ao + kDecH;             // [4] sampling settings (dgpt_sampling), loaded once
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
   const int cr = (int)cluster_rank(), cs = (int)cluster_size(), cid = (int)cluster_id();
   const int gw = cr * kPWarps + w, nw = cs * kPWarps;  // warp index / count inside the cluster
@@ -460,6 +463,8 @@ __global__ void __launch_bounds__(kPThreads, 1) decode_persistent_kernel(DecP p)
   const float scale = rsqrtf((float)kDecH);
   uint64_t seed = p.seed;
   if (p.seed_dev) seed += *p.seed_dev;
+  if (threadIdx.x < 3)  // temperature, top_k (bits), top_p; NULL: 1, 0, 1
+    ss[threadIdx.x] = p.sampling ? reinterpret_cast<const float*>(p.sampling)[threadIdx.x] : (threadIdx.x == 1 ? 0.f : 1.f);
   WPre pre;
   gemv_prefetch(pre, c_dec_layers[0].wqkv, nullptr, 3 * D, C, gw, nw);
   cluster_sync();  // every CTA of the cluster is running before anyone writes into a peer's shared memory
@@ -536,46 +541,11 @@ __global__ void __launch_bounds__(kPThreads, 1) decode_persistent_kernel(DecP p)
     gemv_prefetch(pre, c_dec_layers[0].wqkv, nullptr, 3 * D, C, gw, nw);
     cluster_sync();
     DTS();
-    // ---- next token: argmax, or inverse-CDF sample with u = philox(seed, t, b) (same stream as dgpt_sample) ----
+    // ---- next token: warp_sample_row (sample.cuh) with u = philox(seed, t, b), the same rule and stream as dgpt_sample ----
     if (cr == 0) {
+      const dgpt_sampling sp{ss[0], __float_as_int(ss[1]), ss[2]};
       for (int b = w; b < B; b += kPWarps) {
-        const float* lr = lg + b * V;
-        float mx = -INFINITY;
-        int arg = 0;
-        for (int v = lane; v < V; v += 32) {
-          const float x = lr[v];
-          if (x > mx) { mx = x; arg = v; }
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-          const float om = __shfl_xor_sync(0xffffffffu, mx, o);
-          const int oa = __shfl_xor_sync(0xffffffffu, arg, o);
-          if (om > mx || (om == mx && oa < arg)) { mx = om; arg = oa; }
-        }
-        int choice = arg;
-        if (!p.greedy) {
-          float se = 0.f;
-          for (int v = lane; v < V; v += 32) se += expf(lr[v] - mx);
-          se = warp_sum(se);
-          const u32x4 r = philox4x32_10((uint32_t)(b0 + b), (uint32_t)t, 0x53414d50u, 0u, (uint32_t)seed, (uint32_t)(seed >> 32));
-          const float u = ((float)(r.x >> 8) + 0.5f) * (1.0f / 16777216.0f) * se;
-          float base = 0.f;
-          choice = V - 1;
-          bool done = false;
-          for (int v0 = 0; v0 < V && !done; v0 += 32) {
-            const int v = v0 + lane;
-            const float e = v < V ? expf(lr[v] - mx) : 0.f;
-            float c = e;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-              const float tt = __shfl_up_sync(0xffffffffu, c, o);
-              if (lane >= o) c += tt;
-            }
-            const unsigned hit = __ballot_sync(0xffffffffu, v < V && base + c > u);
-            if (hit) { choice = v0 + __ffs(hit) - 1; done = true; }
-            base += __shfl_sync(0xffffffffu, c, 31);
-          }
-        }
+        const int choice = warp_sample_row(lg + b * V, V, p.greedy != 0, sp, (uint32_t)(b0 + b), (uint32_t)t, seed);
         if (lane == 0) p.seq[(int64_t)(t + 1) * p.B + b0 + b] = (int64_t)choice;
       }
     }
@@ -633,10 +603,10 @@ int64_t dgpt_decode_persistent_scratch_floats(int B, int C, int NH, int F, int V
  * M = batch rows + the KV-streaming attention kernel) is faster: measured crossover between 8 and 16 sequences. */
 int dgpt_decode_persistent_max_batch(void) { return kDecMaxB; }
 
-int dgpt_decode_persistent(const void* const* layers, int nl, const float* tok, const float* pos, const void* wlm,
-                           const float* blm, int64_t* seq, float* scratch, int B, int C, int NH, int H, int F, int V, int ctx,
-                           int t0, int t1, int t_sample, int greedy, uint64_t seed, const uint64_t* seed_dev, int cluster,
-                           void* stream) {
+int dgpt_decode_persistent_ex(const void* const* layers, int nl, const float* tok, const float* pos, const void* wlm,
+                              const float* blm, int64_t* seq, float* scratch, int B, int C, int NH, int H, int F, int V,
+                              int ctx, int t0, int t1, int t_sample, int greedy, uint64_t seed, const uint64_t* seed_dev,
+                              const dgpt_sampling* sampling, int cluster, void* stream) {
   DGPT_DEVICE_OR_RETURN();
   DGPT_REQUIRE(layers && tok && pos && wlm && seq && scratch, "decode_persistent: NULL argument");
   DGPT_REQUIRE(H == kDecH && B >= 1 && nl >= 1 && nl <= kDecMaxL && C % 8 == 0 && F % 8 == 0 && ctx <= 256 && C <= 512 &&
@@ -693,10 +663,10 @@ int dgpt_decode_persistent(const void* const* layers, int nl, const float* tok, 
   p.hbuf = s; s += (int64_t)B * F;
   p.logits = s; s += (int64_t)B * V;
   p.B = B; p.Bc = Bc; p.C = C; p.NH = NH; p.F = F; p.V = V; p.ctx = ctx; p.t0 = t0; p.t1 = t1; p.t_sample = t_sample;
-  p.greedy = greedy; p.seed = seed; p.seed_dev = seed_dev; p.eps = 1e-5f;
+  p.greedy = greedy; p.seed = seed; p.seed_dev = seed_dev; p.sampling = sampling; p.eps = 1e-5f;
   p.probe = clock_probe_buffer();
   const int bm = Bc <= 1 ? 1 : Bc <= 2 ? 2 : Bc <= 4 ? 4 : 8;
-  const size_t smem = ((size_t)bm * (3 * C + D + F + V) + 32 + 8 * kDecH + 2 * kDecH) * sizeof(float);
+  const size_t smem = ((size_t)bm * (3 * C + D + F + V) + 32 + 8 * kDecH + 2 * kDecH + 4) * sizeof(float);
   auto kern = bm == 1 ? decode_persistent_kernel<1> : bm == 2 ? decode_persistent_kernel<2>
               : bm == 4 ? decode_persistent_kernel<4> : decode_persistent_kernel<8>;
   static size_t attr_bytes[4] = {0, 0, 0, 0};
@@ -730,6 +700,14 @@ int dgpt_decode_persistent(const void* const* layers, int nl, const float* tok, 
     return DGPT_E_LAUNCH;
   }
   return check_launch("decode_persistent");
+}
+
+int dgpt_decode_persistent(const void* const* layers, int nl, const float* tok, const float* pos, const void* wlm,
+                           const float* blm, int64_t* seq, float* scratch, int B, int C, int NH, int H, int F, int V, int ctx,
+                           int t0, int t1, int t_sample, int greedy, uint64_t seed, const uint64_t* seed_dev, int cluster,
+                           void* stream) {
+  return dgpt_decode_persistent_ex(layers, nl, tok, pos, wlm, blm, seq, scratch, B, C, NH, H, F, V, ctx, t0, t1, t_sample,
+                                   greedy, seed, seed_dev, nullptr, cluster, stream);
 }
 
 }  // extern "C"

@@ -5,6 +5,7 @@
 // warp per row with float4 accesses; none allocates or synchronises.
 #include "common.cuh"
 #include "ptx.cuh"
+#include "sample.cuh"
 
 namespace dgpt {
 
@@ -862,57 +863,18 @@ __global__ void __launch_bounds__(256) colsum_kernel(const T* __restrict__ X, in
 }
 
 // ---------------------------------------------------------------------------
-// sampler: one warp per sequence
+// sampler: one warp per sequence (the rule is warp_sample_row, sample.cuh)
 // ---------------------------------------------------------------------------
 __global__ void __launch_bounds__(32) sample_kernel(const float* __restrict__ logits, int ld,
                                                     int64_t* __restrict__ seq, int64_t seq_ld, int pos,
                                                     int V, int greedy, uint64_t seed,
-                                                    const uint64_t* __restrict__ seed_dev, uint32_t step) {
+                                                    const uint64_t* __restrict__ seed_dev, uint32_t step,
+                                                    const dgpt_sampling* __restrict__ sampling) {
+  const dgpt_sampling s = sampling ? *sampling : default_sampling();
   if (seed_dev) seed += *seed_dev;
-  const int b = blockIdx.x, lane = threadIdx.x;
-  const float* lr = logits + (int64_t)b * ld;
-  float mx = -INFINITY;
-  int arg = 0x7fffffff;
-  for (int v = lane; v < V; v += 32) {
-    const float l = lr[v];
-    if (l > mx) { mx = l; arg = v; }
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) {
-    const float om = __shfl_xor_sync(0xffffffffu, mx, o);
-    const int oa = __shfl_xor_sync(0xffffffffu, arg, o);
-    if (om > mx || (om == mx && oa < arg)) { mx = om; arg = oa; }
-  }
-  int choice = arg;
-  if (!greedy) {
-    float se = 0.f;
-    for (int v = lane; v < V; v += 32) se += expf(lr[v] - mx);
-    se = warp_sum(se);
-    const u32x4 r = philox4x32_10((uint32_t)b, step, 0x53414d50u /* "SAMP" */, 0u, (uint32_t)seed,
-                                  (uint32_t)(seed >> 32));
-    const float u = ((float)(r.x >> 8) + 0.5f) * (1.0f / 16777216.0f) * se;  // target mass in (0, se)
-    // inverse CDF in vocabulary order, 32 tokens per sweep
-    float base = 0.f;
-    choice = V - 1;
-    bool done = false;
-    for (int v0 = 0; v0 < V && !done; v0 += 32) {
-      const int v = v0 + lane;
-      const float e = v < V ? expf(lr[v] - mx) : 0.f;
-      float c = e;  // inclusive scan
-#pragma unroll
-      for (int o = 1; o < 32; o <<= 1) {
-        const float t = __shfl_up_sync(0xffffffffu, c, o);
-        if (lane >= o) c += t;
-      }
-      const unsigned hit = __ballot_sync(0xffffffffu, v < V && base + c > u);
-      if (hit) {
-        choice = v0 + __ffs(hit) - 1;
-        done = true;
-      }
-      base += __shfl_sync(0xffffffffu, c, 31);
-    }
-  }
-  if (lane == 0) seq[(int64_t)b * seq_ld + pos] = (int64_t)choice;
+  const int b = blockIdx.x;
+  const int choice = warp_sample_row(logits + (int64_t)b * ld, V, greedy != 0, s, (uint32_t)b, step, seed);
+  if (threadIdx.x == 0) seq[(int64_t)b * seq_ld + pos] = (int64_t)choice;
 }
 
 }  // namespace dgpt
@@ -1193,12 +1155,19 @@ int dgpt_colsum(const void* X, int dtype, int M, int N, int ldx, float* out, int
   return check_launch("colsum");
 }
 
-int dgpt_sample(const float* logits, int ld, int64_t* seq, int64_t seq_ld, int pos, int B, int V,
-                int greedy, uint64_t seed, const uint64_t* seed_dev, uint32_t step, void* stream) {
+int dgpt_sample_ex(const float* logits, int ld, int64_t* seq, int64_t seq_ld, int pos, int B, int V,
+                   int greedy, uint64_t seed, const uint64_t* seed_dev, uint32_t step,
+                   const dgpt_sampling* sampling, void* stream) {
   DGPT_DEVICE_OR_RETURN();
   if (B == 0) return DGPT_OK;
-  sample_kernel<<<B, 32, 0, (cudaStream_t)stream>>>(logits, ld, seq, seq_ld, pos, V, greedy, seed, seed_dev, step);
+  sample_kernel<<<B, 32, 0, (cudaStream_t)stream>>>(logits, ld, seq, seq_ld, pos, V, greedy, seed, seed_dev, step,
+                                                    sampling);
   return check_launch("sample");
+}
+
+int dgpt_sample(const float* logits, int ld, int64_t* seq, int64_t seq_ld, int pos, int B, int V,
+                int greedy, uint64_t seed, const uint64_t* seed_dev, uint32_t step, void* stream) {
+  return dgpt_sample_ex(logits, ld, seq, seq_ld, pos, B, V, greedy, seed, seed_dev, step, nullptr, stream);
 }
 
 }  // extern "C"

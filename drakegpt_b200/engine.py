@@ -596,7 +596,7 @@ class Runner:
                 return False
         return C % 8 == 0
 
-    def _decode_persistent(self, seqw, caches, Bn, t_begin, t_end, t_sample, greedy, seed_dev):
+    def _decode_persistent(self, seqw, caches, Bn, t_begin, t_end, t_sample, greedy, seed_dev, sampling=None):
         import ctypes as C_
         from . import _lib
         sp = self.spec
@@ -615,15 +615,20 @@ class Runner:
                   self.f(L["proj"][1]), self.f(L["ffn"][2]), self.f(L["ffn"][4]), caches[li]]
             for j, t in enumerate(ts):
                 ptrs[12 * li + j] = t.data_ptr()
-        _lib.check(lib.dgpt_decode_persistent(ptrs, len(sp["layers"]), tok.data_ptr(), self.f(sp["pos"]).data_ptr(),
-                                              self.w(sp["lm"][0]).data_ptr(), self.f(sp["lm"][1]).data_ptr(),
-                                              seqw.data_ptr(), scratch.data_ptr(), Bn, C, NH, H, F, V, sp["ctx"],
-                                              int(t_begin), int(t_end), int(t_sample), int(bool(greedy)), 0,
-                                              seed_dev.data_ptr(), 0, ops._stream()), "dgpt_decode_persistent")
+        _lib.check(lib.dgpt_decode_persistent_ex(ptrs, len(sp["layers"]), tok.data_ptr(), self.f(sp["pos"]).data_ptr(),
+                                                 self.w(sp["lm"][0]).data_ptr(), self.f(sp["lm"][1]).data_ptr(),
+                                                 seqw.data_ptr(), scratch.data_ptr(), Bn, C, NH, H, F, V, sp["ctx"],
+                                                 int(t_begin), int(t_end), int(t_sample), int(bool(greedy)), 0,
+                                                 seed_dev.data_ptr(), ops._p(sampling), 0, ops._stream()),
+                   "dgpt_decode_persistent_ex")
 
     @torch.no_grad()
-    def generate(self, idx, max_new_tokens, greedy=False, seed=None, use_graphs=None):
-        """(B,t0) int64 -> (B,t0+N) int64.  Sampling (softmax -> multinomial, or argmax) runs on the device.
+    def generate(self, idx, max_new_tokens, greedy=False, seed=None, use_graphs=None, temperature=1.0, top_k=None,
+                 top_p=1.0):
+        """(B,t0) int64 -> (B,t0+N) int64.  Sampling (softmax -> multinomial, or argmax) runs on the device, with
+        optional temperature, top-k and top-p (nucleus) cut-offs (rule: warp_sample_row in csrc/sample.cuh; the
+        defaults draw exactly the plain multinomial).  The settings live in a device buffer beside the sampling seed,
+        so one captured graph serves every setting.
 
         While the window has not slid (t < context_length) every position is one KV-cached decode step.
         Tensor mode, up to 8 sequences: ONE cooperative launch of the persistent decoder (``dgpt_decode_persistent``)
@@ -632,6 +637,7 @@ class Runner:
         ``use_graphs`` (default: tensor mode) -- the sequence buffer, KV caches and sampling seed live in device memory.
         After the slide every token is a full-window recompute (reference semantics, src/model.py:625).
         """
+        ops.check_sampling(temperature, top_k, top_p)
         self._reattach()
         self.flat.refresh_shadow()
         sp = self.spec
@@ -640,13 +646,19 @@ class Runner:
         seed = ops.next_seed() if seed is None else int(seed)
         tok = self.f(sp["tok"])
         V = tok.shape[0]
+        sampling = self.buf("d.sampling", (3,), torch.int32)
+        settings = (float(temperature), top_k, float(top_p))
+        prev = self.__dict__.get("_sampling_in_buf")
+        if prev is None or prev[0] is not sampling or prev[1] != settings:  # upload on change only: a host copy syncs
+            sampling.copy_(ops.sampling_settings(temperature, top_k, top_p))
+            self._sampling_in_buf = (sampling, settings)
         if sp["kind"] == "BigramLM":
             seq = torch.empty((total, Bn), device=self.device, dtype=torch.int64)  # time-major
             seq[:t0].copy_(idx.t())
             logits = self.buf("d.logits", (Bn, V), torch.float32)
             for t in range(t0 - 1, total - 1):
                 ops.raw_embed_fwd(seq[t].view(Bn, 1), tok, None, logits.view(Bn, 1, V))
-                ops.raw_sample(logits, seq[t + 1], 0, greedy, seed, t)
+                ops.raw_sample(logits, seq[t + 1], 0, greedy, seed, t, sampling=sampling)
             return seq.t().contiguous()
         ctx = sp["ctx"]
         if use_graphs is None:
@@ -667,31 +679,31 @@ class Runner:
         if self._persistent_decode_ok(Bn) and n_in > 0:
             # small batch: ONE launch (a thread-block cluster per sequence) walks every in-window position (all layers, KV append, attention,
             # LM head, sampling) -- no per-token launches at all
-            self._decode_persistent(seqw, caches, Bn, 0, n_in, t0 - 1, greedy, sample_seed)
+            self._decode_persistent(seqw, caches, Bn, 0, n_in, t0 - 1, greedy, sample_seed, sampling)
             n_done = n_in
         else:
             n_done = 0
 
-        def step_kernels(t, sampling, greedy_flag):
+        def step_kernels(t, draw, greedy_flag):
             x = self._decode_token(seqw[t], t, caches)
-            if sampling:
+            if draw:
                 xin = x if x.dtype == self.at else ops.raw_dropout_scale(x, self.buf("d.xl", x.shape))
                 self._gemm(xin, self.w(sp["lm"][0]), logits, bias=self.f(sp["lm"][1]))
-                ops.raw_sample(logits, seqw[t + 1], 0, greedy_flag, 0, t, seed_dev=sample_seed)
+                ops.raw_sample(logits, seqw[t + 1], 0, greedy_flag, 0, t, seed_dev=sample_seed, sampling=sampling)
 
         for t in range(n_done, n_in):
-            sampling = t >= t0 - 1
+            draw = t >= t0 - 1
             if not use_graphs:
-                step_kernels(t, sampling, greedy)
+                step_kernels(t, draw, greedy)
                 continue
-            key = (Bn, t, sampling, bool(greedy), self._flat_gen)
+            key = (Bn, t, draw, bool(greedy), self._flat_gen)
             g = graphs.get(key)
             if g is None:
-                step_kernels(t, sampling, greedy)  # warm-up: allocates workspaces, loads kernels
+                step_kernels(t, draw, greedy)  # warm-up: allocates workspaces, loads kernels
                 torch.cuda.synchronize(self.device)
                 g = torch.cuda.CUDAGraph()
                 with torch.cuda.graph(g):
-                    step_kernels(t, sampling, greedy)
+                    step_kernels(t, draw, greedy)
                 graphs[key] = g
             else:
                 g.replay()
@@ -704,5 +716,5 @@ class Runner:
                 win = seq[t - ctx + 1: t + 1].t().contiguous()
                 full, _ = self.forward(win)
                 last = full.view(Bn, ctx, V)[:, -1, :]
-                ops.raw_sample(last, seq[t + 1], 0, greedy, seed, t)
+                ops.raw_sample(last, seq[t + 1], 0, greedy, seed, t, sampling=sampling)
         return seq[:total].t().contiguous()

@@ -13,7 +13,8 @@ Execution:
     (also reachable as ``model.runner()`` for the graph-captured training step);
   * ``generate`` always runs the Runner: KV-cached decode with on-device sampling
     until the context window slides, full-window recompute afterwards.  ``greedy=True``
-    (argmax) is an extension used by the parity tests (SURVEY Q13).
+    (argmax) is an extension used by the parity tests (SURVEY Q13); so are ``temperature``,
+    ``top_k`` and ``top_p``, whose defaults keep the reference's plain multinomial.
 """
 from collections import OrderedDict
 
@@ -111,9 +112,15 @@ class _LM(nn.Module):
         return flat, ops.cross_entropy(flat, targets.view(B * T))
 
     @torch.no_grad()
-    def generate(self, idx, max_new_tokens, greedy=False, seed=None):
+    def generate(self, idx, max_new_tokens, greedy=False, seed=None, temperature=1.0, top_k=None, top_p=1.0):
+        """Continue ``idx`` (B, t0) by ``max_new_tokens`` tokens.  ``temperature`` (> 0) divides the logits, ``top_k``
+        (None or >= 1) keeps the k most likely tokens (ties at the k-th logit kept), ``top_p`` (in (0, 1]) keeps the
+        smallest most-likely prefix whose mass reaches it.  The defaults are the reference's softmax -> multinomial;
+        ``greedy=True`` (argmax) ignores them.  ``seed`` fixes the draw."""
+        ops.check_sampling(temperature, top_k, top_p)
         self._check(idx)
-        return self.runner().generate(idx, max_new_tokens, greedy=greedy, seed=seed)
+        return self.runner().generate(idx, max_new_tokens, greedy=greedy, seed=seed, temperature=temperature,
+                                      top_k=top_k, top_p=top_p)
 
 
 class BigramLM(_LM):

@@ -10,6 +10,9 @@ Nothing here computes with PyTorch ops: torch supplies device memory, streams
 and the autograd tape only.
 """
 import ctypes as C
+import math
+import numbers
+import struct
 
 import torch
 
@@ -299,10 +302,37 @@ def raw_counter_add(ctr, delta=1):
     check(_lib.lib().dgpt_counter_add(_p(ctr), int(delta), _stream()), "dgpt_counter_add")
 
 
-def raw_sample(logits, seq, pos, greedy, seed, step, seed_dev=None):
+def check_sampling(temperature=1.0, top_k=None, top_p=1.0):
+    """Validate generate()'s sampling settings; raise ValueError before anything is launched."""
+    if isinstance(temperature, bool) or not isinstance(temperature, numbers.Real) \
+            or not math.isfinite(temperature) or temperature <= 0:
+        raise ValueError(f"temperature must be a finite number > 0, got {temperature!r}")
+    if top_k is not None and (isinstance(top_k, bool) or not isinstance(top_k, numbers.Integral) or top_k < 1):
+        raise ValueError(f"top_k must be None or an int >= 1, got {top_k!r}")
+    if isinstance(top_p, bool) or not isinstance(top_p, numbers.Real) or not 0 < top_p <= 1:
+        raise ValueError(f"top_p must be in (0, 1], got {top_p!r}")
+
+
+def sampling_settings(temperature=1.0, top_k=None, top_p=1.0):
+    """Host int32[3] tensor laid out as the C-ABI's dgpt_sampling {float temperature; int32 top_k; float top_p}
+    (top_k 0 = off).  Copy it into a device buffer and hand that to raw_sample / the persistent decoder.  The
+    temperature is stored as float32 within [smallest normal, largest finite], so 1 / temperature stays finite."""
+    check_sampling(temperature, top_k, top_p)
+    t = min(max(float(temperature), 1.1754944e-38), 3.4028234e38)
+    k = 0 if top_k is None else min(int(top_k), 2 ** 31 - 1)
+    return torch.frombuffer(bytearray(struct.pack("<fif", t, k, float(top_p))), dtype=torch.int32).clone()
+
+
+def raw_sample(logits, seq, pos, greedy, seed, step, seed_dev=None, sampling=None):
+    """Next token of every row of ``logits`` into ``seq[b, pos]``.  ``sampling``: device int32[3] buffer filled from
+    ``sampling_settings`` (temperature, top-k, top-p), or None for the plain softmax -> multinomial draw."""
     Bn, V = logits.shape
-    check(_lib.lib().dgpt_sample(_p(logits), logits.stride(0), _p(seq), seq.stride(0), pos, Bn, V, int(greedy),
-                                 int(seed), _p(seed_dev), int(step), _stream()), "dgpt_sample")
+    if sampling is not None:
+        _need_cuda(sampling)
+        if sampling.dtype != torch.int32 or sampling.numel() != 3 or not sampling.is_contiguous():
+            raise ValueError("raw_sample: sampling must be a contiguous int32[3] device tensor from sampling_settings")
+    check(_lib.lib().dgpt_sample_ex(_p(logits), logits.stride(0), _p(seq), seq.stride(0), pos, Bn, V, int(greedy),
+                                    int(seed), _p(seed_dev), int(step), _p(sampling), _stream()), "dgpt_sample_ex")
 
 
 # --------------------------------------------------------------------------- #

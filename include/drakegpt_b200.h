@@ -322,9 +322,33 @@ int dgpt_counter_add(uint64_t* ctr, uint64_t delta, void* stream);
  *   greedy != 0: argmax (lowest index wins ties, like torch.argmax)
  *   else inverse-CDF sample with u = philox(seed + *seed_dev, step, b)  (seed_dev may be NULL).
  * Writes the token to seq[b*seq_ld + pos] (int64).
+ *
+ * dgpt_sample_ex also takes a DEVICE pointer to one dgpt_sampling struct;
+ * NULL gives dgpt_sample's plain multinomial.  For one row l[0..V):
+ *   1. top_k >= 1: keep v iff l[v] >= the k-th largest logit (ties kept);
+ *      top_k <= 0 or >= V: off.
+ *   2. e[v] = exp((l[v] - max) * (1 / temperature)) over the kept tokens,
+ *      0 for the others.
+ *   3. top_p < 1: order by e descending (lower index first on ties); keep v
+ *      iff the sum of e over the tokens ahead of it is < top_p * sum(e).
+ *   4. u = ((r.x >> 8) + 0.5) / 2^24 * (kept mass), r = philox4x32_10(b,
+ *      step, 0x53414d50, 0; seed): the first v in vocabulary order whose
+ *      inclusive cumulative kept mass is > u.
+ * greedy ignores the settings (every filtered set contains the argmax).  With
+ * temperature 1 and both cut-offs off the draw is exactly dgpt_sample's.  The
+ * settings live in device memory so that one captured CUDA graph serves all.
+ * The caller validates them (temperature > 0, 0 < top_p <= 1).
  * ------------------------------------------------------------------------- */
+typedef struct dgpt_sampling {
+  float temperature;
+  int32_t top_k;
+  float top_p;
+} dgpt_sampling;
 int dgpt_sample(const float* logits, int ld, int64_t* seq, int64_t seq_ld, int pos, int B, int V,
                 int greedy, uint64_t seed, const uint64_t* seed_dev, uint32_t step, void* stream);
+int dgpt_sample_ex(const float* logits, int ld, int64_t* seq, int64_t seq_ld, int pos, int B, int V,
+                   int greedy, uint64_t seed, const uint64_t* seed_dev, uint32_t step,
+                   const dgpt_sampling* sampling, void* stream);
 
 /* ------------------------------------------------------------------------- *
  * KV-cached generation (tensor mode, head size 64, context <= 256) -- the
@@ -341,7 +365,7 @@ int dgpt_sample(const float* logits, int ld, int64_t* seq, int64_t seq_ld, int p
  *   LayerNorm + packed QKV matrix-vector product + KV append, attention,
  *   projection + residual, LayerNorm + FFN (+ReLU) + residual, then the LM head
  *   (ln_f is not applied, src/model.py:598-599) and the next token -- argmax
- *   (greedy != 0) or the same inverse-CDF / Philox stream as dgpt_sample
+ *   (greedy != 0) or the same draw as dgpt_sample / dgpt_sample_ex
  *   (step = t) -- written to seq[(t+1)*B + b] for t >= t_sample.
  *   One thread-block CLUSTER (16 CTAs; `cluster` = 4 / 8 / 16, 0 = default) per
  *   group of <= 8 sequences, hardware cluster barriers between the phases, the
@@ -362,6 +386,12 @@ int dgpt_decode_persistent(const void* const* layers, int nl, const float* tok, 
                            int C, int NH, int H, int F, int V, int ctx, int t0, int t1, int t_sample,
                            int greedy, uint64_t seed, const uint64_t* seed_dev, int cluster,
                            void* stream);
+/* the same with the sampling settings of dgpt_sample_ex (device pointer, NULL = plain multinomial) */
+int dgpt_decode_persistent_ex(const void* const* layers, int nl, const float* tok, const float* pos,
+                              const void* wlm, const float* blm, int64_t* seq, float* scratch, int B,
+                              int C, int NH, int H, int F, int V, int ctx, int t0, int t1,
+                              int t_sample, int greedy, uint64_t seed, const uint64_t* seed_dev,
+                              const dgpt_sampling* sampling, int cluster, void* stream);
 
 #ifdef __cplusplus
 }
