@@ -21,6 +21,7 @@ EXPORTS = [
     "dgpt_ipc_export", "dgpt_ipc_open", "dgpt_ipc_close", "dgpt_peer_copy", "dgpt_dp_adamw",
     "dgpt_decode_attn", "dgpt_decode_persistent", "dgpt_decode_persistent_scratch_floats",
     "dgpt_decode_persistent_max_batch", "dgpt_sample_ex", "dgpt_decode_persistent_ex",
+    "dgpt_decode_persistent_supported",
 ]
 
 
@@ -105,6 +106,7 @@ def _declare(lib):
         "dgpt_sample_ex": [vp, i32, vp, i64, i32, i32, i32, i32, u64, vp, u32, vp, vp],
         "dgpt_decode_persistent_ex": [C.POINTER(C.c_void_p), i32, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32,
                                       i32, i32, i32, i32, i32, u64, vp, vp, i32, vp],
+        "dgpt_decode_persistent_supported": [i32, i32, i32, i32, i32, i32, i32, i32, i32],
     }
     for name, args in sig.items():
         fn = getattr(lib, name)

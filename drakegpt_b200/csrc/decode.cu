@@ -554,6 +554,38 @@ __global__ void __launch_bounds__(kPThreads, 1) decode_persistent_kernel(DecP p)
   cluster_sync();  // no CTA exits while a peer may still write into its shared memory
 }
 
+// cluster <= 0: the launch's default, 16 CTAs (DGPT_DECODE_CLUSTER overrides it; read once per process)
+static int decode_cluster_size(int cluster) {
+  if (cluster > 0) return cluster;
+  static int env_cluster = -1;
+  if (env_cluster < 0) { const char* e = getenv("DGPT_DECODE_CLUSTER"); env_cluster = e ? atoi(e) : 0; }
+  return env_cluster > 0 ? env_cluster : 16;
+}
+
+// The shapes decode_persistent_kernel handles: the one rule behind dgpt_decode_persistent_supported and the launch.
+// report: say why a shape is refused (dgpt_last_error).
+static bool decode_persistent_shape_ok(int B, int nl, int C, int NH, int H, int F, int V, int ctx, int cluster, bool report) {
+#define DEC_GATE(cond, ...) do { if (!(cond)) { if (report) set_error(__VA_ARGS__); return false; } } while (0)
+  // ln_rows_smem holds a row in 4 float4 per lane (C <= 512); the 6-chunk matrix-vector form reads K <= 1536;
+  // cta_attend gives each cached key a thread of its own (context <= 256)
+  DEC_GATE(H == kDecH && B >= 1 && nl >= 1 && nl <= kDecMaxL && NH >= 1 && V >= 1 && C >= 8 && F >= 8 && C % 8 == 0 &&
+               F % 8 == 0 && ctx >= 1 && ctx <= 256 && C <= 512 && F <= 1536 && NH * kDecH <= 1536,
+           "decode_persistent: head size 64, <= 8 layers, C <= 512 and F <= 1536 multiples of 8, context <= 256 "
+           "(H=%d layers=%d C=%d F=%d ctx=%d)", H, nl, C, F, ctx);
+  cluster = decode_cluster_size(cluster);
+  DEC_GATE(cluster == 16 || cluster == 8 || cluster == 4, "decode_persistent: cluster size %d (4, 8 or 16)", cluster);
+  {
+    // every weight row of a phase must fit the per-warp register budget: 12 rows of K <= 512, 4 rows of K <= 1536
+    const int nwarps = cluster * kPWarps, D3 = 3 * NH * kDecH;
+    const int r_c = C <= 512 ? 12 : 4, r_f = F <= 512 ? 12 : 4, r_d = NH * kDecH <= 512 ? 12 : 4;
+    DEC_GATE(D3 <= r_c * nwarps && F <= r_c * nwarps && V <= r_c * nwarps && C <= r_d * nwarps && C <= r_f * nwarps,
+             "decode_persistent: model too wide for a cluster of %d CTAs (3D=%d F=%d C=%d V=%d)", cluster, D3, F, C, V);
+  }
+  DEC_GATE(B <= kDecMaxB, "decode_persistent: batch %d > %d (use the launch-per-kernel path)", B, kDecMaxB);
+#undef DEC_GATE
+  return true;
+}
+
 }  // namespace dgpt
 
 using namespace dgpt;
@@ -603,37 +635,25 @@ int64_t dgpt_decode_persistent_scratch_floats(int B, int C, int NH, int F, int V
  * M = batch rows + the KV-streaming attention kernel) is faster: measured crossover between 8 and 16 sequences. */
 int dgpt_decode_persistent_max_batch(void) { return kDecMaxB; }
 
+int dgpt_decode_persistent_supported(int B, int nl, int C, int NH, int H, int F, int V, int ctx, int cluster) {
+  return decode_persistent_shape_ok(B, nl, C, NH, H, F, V, ctx, cluster, false) ? 1 : 0;
+}
+
 int dgpt_decode_persistent_ex(const void* const* layers, int nl, const float* tok, const float* pos, const void* wlm,
                               const float* blm, int64_t* seq, float* scratch, int B, int C, int NH, int H, int F, int V,
                               int ctx, int t0, int t1, int t_sample, int greedy, uint64_t seed, const uint64_t* seed_dev,
                               const dgpt_sampling* sampling, int cluster, void* stream) {
   DGPT_DEVICE_OR_RETURN();
   DGPT_REQUIRE(layers && tok && pos && wlm && seq && scratch, "decode_persistent: NULL argument");
-  DGPT_REQUIRE(H == kDecH && B >= 1 && nl >= 1 && nl <= kDecMaxL && C % 8 == 0 && F % 8 == 0 && ctx <= 256 && C <= 512 &&
-                   F <= 1536 && NH * kDecH <= 1536,
-               "decode_persistent: head size 64, <= 8 layers, C <= 512 and F <= 1536 multiples of 8, context <= 256 "
-               "(H=%d layers=%d C=%d F=%d ctx=%d)", H, nl, C, F, ctx);
+  if (!decode_persistent_shape_ok(B, nl, C, NH, H, F, V, ctx, cluster, true)) return DGPT_E_ARG;
   DGPT_REQUIRE(0 <= t0 && t0 <= t1 && t1 <= ctx, "decode_persistent: positions [%d, %d) outside the context %d", t0, t1, ctx);
   if (t0 == t1) return DGPT_OK;
-  if (cluster <= 0) {
-    static int env_cluster = -1;
-    if (env_cluster < 0) { const char* e = getenv("DGPT_DECODE_CLUSTER"); env_cluster = e ? atoi(e) : 0; }
-    cluster = env_cluster > 0 ? env_cluster : 16;
-  }
-  DGPT_REQUIRE(cluster == 16 || cluster == 8 || cluster == 4, "decode_persistent: cluster size %d (4, 8 or 16)", cluster);
-  {
-    // every weight row of a phase must fit the per-warp register budget: 12 rows of K <= 512, 4 rows of K <= 1536
-    const int nwarps = cluster * kPWarps, D3 = 3 * NH * kDecH;
-    const int r_c = C <= 512 ? 12 : 4, r_f = F <= 512 ? 12 : 4, r_d = NH * kDecH <= 512 ? 12 : 4;
-    DGPT_REQUIRE(D3 <= r_c * nwarps && F <= r_c * nwarps && V <= r_c * nwarps && C <= r_d * nwarps && C <= r_f * nwarps,
-                 "decode_persistent: model too wide for a cluster of %d CTAs (3D=%d F=%d C=%d V=%d)", cluster, D3, F, C, V);
-  }
+  cluster = decode_cluster_size(cluster);
   // one cluster per sequence while the clusters can all be resident at once (16 CTAs of one cluster need 16 SMs of
   // ONE GPC: 4 co-resident clusters measured on B200), else several sequences per cluster
   static int env_nc = -1;
   if (env_nc < 0) { const char* e = getenv("DGPT_DECODE_CLUSTERS"); env_nc = e ? atoi(e) : 0; }
   const int max_clusters = env_nc > 0 ? env_nc : 4;
-  DGPT_REQUIRE(B <= kDecMaxB, "decode_persistent: batch %d > %d (use the launch-per-kernel path)", B, kDecMaxB);
   const int nclusters = min(B, max_clusters);
   const int Bc = ceil_div(B, nclusters);
   DecP p;

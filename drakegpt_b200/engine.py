@@ -577,7 +577,9 @@ class Runner:
         context <= 256.  It is used while every sequence gets a 16-CTA cluster of its own (<= 4 sequences: 134 us per
         token against 187-191 us for the per-position graphs); with two sequences per cluster (5-8) it measures 216 us
         against 191-193 us, so those batches take the graph path.  DGPT_DECODE_PERSISTENT=0 turns it off,
-        DGPT_DECODE_PERSISTENT=force uses it up to the kernel's limit of 8 sequences (A/B runs, tests)."""
+        DGPT_DECODE_PERSISTENT=force uses it up to the kernel's limit of 8 sequences (A/B runs, tests).
+        The shape limits (width, layers, context, cluster budget) are the kernel's own, dgpt_decode_persistent_supported:
+        a model outside them takes the per-position path."""
         import os
         from . import _lib
         sp = self.spec
@@ -587,14 +589,19 @@ class Runner:
         limit = int(_lib.lib().dgpt_decode_persistent_max_batch())
         if not (1 <= Bn <= (limit if env == "force" else min(limit, 4))):
             return False
-        if sp["ctx"] is None or sp["ctx"] > 256 or not (1 <= len(sp["layers"]) <= 8):
+        if sp["ctx"] is None or not sp["layers"]:
             return False
-        C = self.f(sp["tok"]).shape[1]
+        V, C = self.f(sp["tok"]).shape
         for L in sp["layers"]:
-            if (L["H"] != 64 or L["ln1"] is None or L["ln2"] is None or L["proj"] is None or not L["residual"]
+            if (L["ln1"] is None or L["ln2"] is None or L["proj"] is None or not L["residual"]
                     or L["ffn"] is None or L["ffn"][0] != "mlp" or L["NH"] * L["H"] != C):
                 return False
-        return C % 8 == 0
+        # the kernel takes one (NH, H, F) for every layer
+        L0 = sp["layers"][0]
+        F = self.f(L0["ffn"][1]).shape[0]
+        if any((L["NH"], L["H"], self.f(L["ffn"][1]).shape[0]) != (L0["NH"], L0["H"], F) for L in sp["layers"]):
+            return False
+        return ops.decode_persistent_supported(Bn, len(sp["layers"]), C, L0["NH"], L0["H"], F, V, sp["ctx"])
 
     def _decode_persistent(self, seqw, caches, Bn, t_begin, t_end, t_sample, greedy, seed_dev, sampling=None):
         import ctypes as C_

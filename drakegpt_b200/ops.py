@@ -177,6 +177,13 @@ def raw_decode_attn(q, k, v, o, NH, H, scale):
     return o
 
 
+def decode_persistent_supported(B, nl, C, NH, H, F, V, ctx, cluster=0):
+    """Whether the one-launch persistent decoder takes this shape (dgpt_decode_persistent_supported; cluster 0 =
+    the cluster size the launch would use).  Host only: needs no device."""
+    return bool(_lib.lib().dgpt_decode_persistent_supported(int(B), int(nl), int(C), int(NH), int(H), int(F), int(V),
+                                                             int(ctx), int(cluster)))
+
+
 def raw_embed_fwd(idx, tok, pos, x, pos_offset=0):
     _need_cuda(idx, tok, x)
     B, T = idx.shape

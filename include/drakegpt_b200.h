@@ -375,12 +375,21 @@ int dgpt_sample_ex(const float* logits, int ld, int64_t* seq, int64_t seq_ld, in
  *     wproj [C,D], w1 [F,C], w2 [C,F] (bf16), ln1 gamma/beta, ln2 gamma/beta,
  *     proj bias, b1, b2 (fp32), KV cache [B, ctx, 3D] (bf16, sequence-major).
  *   scratch: dgpt_decode_persistent_scratch_floats() floats.
+ * dgpt_decode_persistent_supported: 1 if dgpt_decode_persistent takes this
+ *   shape, else 0 (host only, needs no device).  The launch refuses exactly the
+ *   shapes this refuses: head size 64, 1 <= B <= 8, 1 <= nl <= 8, C <= 512 and
+ *   F <= 1536 (multiples of 8), NH * 64 <= 1536, ctx <= 256, cluster 4 / 8 / 16
+ *   (<= 0: the size the launch would use), and every matrix-vector phase's
+ *   rows (3D, F, V of K = C; C of K = D and of K = F) within the cluster's
+ *   register budget: 12 rows per warp for K <= 512, 4 for K <= 1536.
  * ------------------------------------------------------------------------- */
 int dgpt_decode_attn(const void* q, const void* k, const void* v, void* o, int64_t q_bs, int64_t k_bs,
                      int64_t k_rs, int64_t v_bs, int64_t v_rs, int64_t o_bs, int B, int NH, int H,
                      int nk, float scale, void* stream);
 int64_t dgpt_decode_persistent_scratch_floats(int B, int C, int NH, int F, int V);
 int dgpt_decode_persistent_max_batch(void);
+int dgpt_decode_persistent_supported(int B, int nl, int C, int NH, int H, int F, int V, int ctx,
+                                     int cluster);
 int dgpt_decode_persistent(const void* const* layers, int nl, const float* tok, const float* pos,
                            const void* wlm, const float* blm, int64_t* seq, float* scratch, int B,
                            int C, int NH, int H, int F, int V, int ctx, int t0, int t1, int t_sample,

@@ -242,3 +242,29 @@ def test_wgrad_split_k_follows_the_tile_policy():
     assert Runner._splits(C, F, M, sm) == 4            # FFN2 wgrad without a column sum: 3 x 12 tiles of 128
     assert Runner._splits(C, F, M, sm, colsum=True) == 8   # with the bias gradient riding on it: 3 x 6 tiles of 256
     assert Runner._splits(80, C, 64, sm) == 1          # never more splits than 512-deep K slices
+
+
+def test_persistent_decoder_shape_gate_boundaries():
+    """dgpt_decode_persistent_supported (host only): each limit of decode_persistent_kernel passes at its value and
+    fails one step past it.  Base shape: the scaled TransformerLM (C=384, 6 heads, F=1536, V=80, 6 layers, ctx 256)."""
+    from drakegpt_b200 import ops
+    base = dict(B=4, nl=6, C=384, NH=6, H=64, F=1536, V=80, ctx=256, cluster=16)
+
+    def ok(**kw):
+        a = dict(base, **kw)
+        return ops.decode_persistent_supported(a["B"], a["nl"], a["C"], a["NH"], a["H"], a["F"], a["V"], a["ctx"],
+                                               a["cluster"])
+
+    assert ok() and ok(cluster=0)  # 0: the default cluster of 16
+    for name, at, past in [("C", 512, 520), ("F", 1536, 1544), ("V", 1536, 1537), ("nl", 8, 9), ("ctx", 256, 257),
+                           ("B", 8, 9)]:
+        assert ok(**{name: at}) and not ok(**{name: past}), (name, at, past)
+    assert ok(C=512, NH=8, F=1536) and not ok(C=512, NH=8, F=2048)  # TransformerLM(80, 512, 256, 8, L): F = 4 C
+    assert ok(C=256, NH=8, F=1024)                       # D = NH * 64 != C
+    assert ok(nl=1, B=1) and not ok(nl=0) and not ok(B=0)
+    assert not ok(H=32) and not ok(C=388) and not ok(F=1540)
+    # the row budget: 3D (K = C) <= 12 rows x 128 warps at cluster 16, 4 rows x 64 warps of K <= 1536 at cluster 8
+    assert ok(C=512, NH=8) and not ok(C=512, NH=9)
+    assert ok(cluster=8, C=128, NH=2, F=512, V=80) and not ok(cluster=8)
+    assert ok(cluster=4, C=64, NH=1, F=256, V=80) and not ok(cluster=4, C=128, NH=2, F=512, V=80)
+    assert not ok(cluster=2) and not ok(cluster=32)
